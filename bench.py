@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- contrastive-path pixels/sec of the CSS representation-space hot path on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload voc321_mix|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload voc321_mix|...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one pass of the four-stage path over one synthetic batch per GPU (SURVEY.md 8(d) `t_path`):
@@ -53,7 +53,34 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="launch every step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--cpu-budget-s", type=float, default=float(os.environ.get("CSS_CPU_BUDGET_S", 240)))
     ap.add_argument("--no-gpu-eager-reference", action="store_true", help="skip the reference-on-this-GPU context line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy in float32; "
+                         f"an array of more than {DUMP_MAX_ELEMS} elements is reduced to a fixed seeded sample of its flat indices")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+DUMP_MAX_ELEMS = 1 << 21      # 8 MB per array: at most 4 maps + grad_rep + prob + loss + prototypes stay under 64 MB
+DUMP_SEED = 20240607
+
+
+def dump_outputs(outputs, out_dir):
+    """Copies the named device tensors to DIR/<name>.npy as float32.  A larger array becomes the elements at
+    DUMP_MAX_ELEMS flat (logical, row-major) indices drawn without replacement from a generator seeded with DUMP_SEED and
+    sorted, so the sample depends only on the array's size and two builds write comparable files."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def make_inputs(cfg, rank):
@@ -411,22 +438,22 @@ def main():
                                   seed=3407 + rank).to(dev)
 
     def step(t, rep_for_loss=None):
-        """one pass of the path on device-resident tensors `t`; returns (loss, grad_rep, maps the augmentation receives).
+        """one pass of the path on device-resident tensors `t`; returns (loss, grad_rep, {name: map the augmentation receives},
+        prob_all or None where prob is an input).
         rep_for_loss: what DistributedDataParallel(find_unused_parameters=True) hands the loss instead of rep_all (a clone)."""
-        maps = ()
         if strategy == "ori":
             conf, lab = css_b200.ops.cls_pseudo_label(t["pred_u"], (H, W))
-            prob = t["prob_ori"]
-            maps = (lab, conf)
+            prob, prob_out = t["prob_ori"], None
+            maps = {"label_cls": lab, "conf_cls": conf}
         else:
             o = css_b200.ops.pseudo_labels(t["rep_u"], t["pred_u"], protos, temp, (H, W), fuse="mix" if strategy == "mix" else "none")
-            prob = css_b200.ops.proto_softmax_sim(t["rep_all"], protos, temp)
-            maps = (o["fused"], o["conf_cls"], o["conf_rep"]) if strategy == "mix" else \
-                (o["label_cls"], o["label_rep"], o["conf_cls"], o["conf_rep"])
+            prob = prob_out = css_b200.ops.proto_softmax_sim(t["rep_all"], protos, temp)
+            names = ("fused", "conf_cls", "conf_rep") if strategy == "mix" else ("label_cls", "label_rep", "conf_cls", "conf_rep")
+            maps = {k: o[k] for k in names}
         rep = (t["rep_all"] if rep_for_loss is None else rep_for_loss).detach().requires_grad_(True)
         loss = crit(rep, t["label"], t["mask"], prob, protos)
         (grad,) = torch.autograd.grad(loss, rep)
-        return loss, grad, maps
+        return loss, grad, maps, prob_out
 
     def barrier():
         if world > 1:
@@ -435,7 +462,7 @@ def main():
 
     # ---- warm-up ------------------------------------------------------------------------------------------------
     for _ in range(max(args.warmup, 3)):
-        loss, grad, _ = step(gpu)
+        loss, grad, _, _ = step(gpu)
     barrier()
     meta = crit.last["ws"].meta.cpu().numpy()
     V = int(meta[_lib.META_V])
@@ -492,8 +519,8 @@ def main():
     def run_step():
         if graph is not None:
             graph.replay()
-        else:
-            step(gpu)
+            return graph_out
+        return step(gpu)
 
     # ---- timed region: device-resident inputs ------------------------------------------------------------------------
     sampler = ClockSampler(physical_gpu_index(local_rank))
@@ -510,11 +537,16 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         run_step()
+    out = run_step()                         # only the last step's results are kept (what --dump-outputs writes)
     e1.record()
     barrier()
     elapsed_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:      # before anything below runs the path again (prototypes are updated in place)
+        loss_t, grad_t, maps_t, prob_t = out
+        dump_outputs({"loss": loss_t, "grad_rep": grad_t, **maps_t, **({"prob_all": prob_t} if prob_t is not None else {}),
+                      "prototypes": protos}, args.dump_outputs)
     comm1 = reducer.stats() if comm0 is not None else None
     launches = lib.css_launch_count() - launches0 if graph is None else launches_per_step * args.steps
     clocks = sampler.stop()
@@ -627,8 +659,8 @@ def main():
         except Exception as e:
             sys.stderr.write(f"bench: e2e graph capture failed ({e!r}); eager\n")
             e2e_graphs = [None, None]
-    _, _, maps0 = step(staged[0])
-    host_maps = [torch.empty(m.shape, dtype=m.dtype).pin_memory() for m in maps0]
+    _, _, maps0, _ = step(staged[0])
+    host_maps = [torch.empty(m.shape, dtype=m.dtype).pin_memory() for m in maps0.values()]
     d2h = 4 + sum(m.numel() * m.element_size() for m in host_maps)
 
     def upload(i):
@@ -650,10 +682,10 @@ def main():
             torch.cuda.current_stream().wait_event(ready[s_])
             if e2e_graphs[s_] is not None:
                 e2e_graphs[s_][0].replay()
-                loss, _, maps = e2e_graphs[s_][1]
+                loss, _, maps, _ = e2e_graphs[s_][1]
             else:
-                loss, grad, maps = step(staged[s_])
-            for hm, m in zip(host_maps, maps):      # what the reference flow ships to the host for the PIL augmentation
+                loss, grad, maps, _ = step(staged[s_])
+            for hm, m in zip(host_maps, maps.values()):      # what the reference flow ships to the host for the PIL augmentation
                 hm.copy_(m, non_blocking=True)
             done[s_].record()
             float(loss.item())                # D2H read of the step's result (synchronises; the map copies precede it in stream order)

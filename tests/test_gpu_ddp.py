@@ -196,7 +196,7 @@ def _label_onehot_2(inputs, num_class):                     # generalframeworks/
 
 
 @pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "generalframeworks")) or not os.path.exists(os.path.join(REF, "mix_label.py")),
-                    reason="the reference did not travel to this box (baseline/_ref is made by __graft_entry__.build() where /root/reference exists)")
+                    reason="no reference checkout in baseline/_ref or at CSS_REFERENCE_ROOT")
 def test_unmodified_mix_label_train_under_ddp(world1):
     """The reference's OWN train() (mix_label.py:154-197, imported unmodified) driving the css_b200 classes that install()
     swapped in, with the reference's DeepLabv3+ (torchvision ResNet-50 trunk to keep the test light), its PIL augmentation and

@@ -1,15 +1,15 @@
-"""css_b200.install.install() against an unmodified reference checkout (only where the reference tree exists: the build
-container; on the GPU box this test skips).  Checks that the names the scripts import are replaced and that the shells are
+"""css_b200.install.install() against an unmodified reference checkout (WangChangqi98/CSS), named by $CSS_REFERENCE_ROOT;
+without one this test skips.  Checks that the names the scripts import are replaced and that the shells are
 wired to the reference's own network / augmentation functions."""
 import os
 import sys
 
 import pytest
 
-REF = os.environ.get("CSS_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("CSS_REFERENCE_ROOT", "")
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "generalframeworks")), reason="reference tree not present")
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "generalframeworks")), reason="no reference checkout: set CSS_REFERENCE_ROOT")
 def test_install_patches_reference_modules():
     import torch
     import torch.distributed as dist
