@@ -63,6 +63,8 @@ SIGNATURES = {
     "css_stats_allreduce": (c_int, [P, P, P, c_int, c_int, c_int, c_int, P]),
     "css_aug_index": (c_int, [P, c_int, c_int, c_int, c_int, P, P, P]),
     "css_aug_maps": (c_int, [P, P, c_int, P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, P, P, P, P, P]),
+    "css_aug_image_workspace_bytes": (ctypes.c_size_t, [c_int, c_int, c_int]),
+    "css_aug_image": (c_int, [P, c_int, c_int, c_int, P, P, P, c_int, c_int, P, ctypes.c_size_t, P, P]),
     "css_cut_mix": (c_int, [P, P, P, P, P, P, P, P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, P, P]),
     "css_threshold_glue": (c_int, [P, P, P, c_float, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, P, P]),
 }

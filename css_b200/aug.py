@@ -1,13 +1,14 @@
-"""GPU-resident hand-off of the pseudo-label / confidence maps through the augmentation (SURVEY.md 8(f)-2).
+"""GPU-resident augmentation of the image and of the pseudo-label / confidence maps (SURVEY.md 8(f)-2).
 
-The reference sends every map of every image GPU -> PIL -> GPU twice per step (dataset_helpers/VOC.py:284-302 into
-transform_* :64-274 and back, driven by batch_transform_* :312-352) and mixes images with a Python loop of small
-kernels behind four all_gathers (generate_cut_gather_* :354-477).  For the maps, that trip is index arithmetic plus
-an 8-bit quantisation, so here
+The reference sends every image and map of every image GPU -> PIL -> GPU twice per step (dataset_helpers/VOC.py:284-302
+into transform_* :64-274 and back, driven by batch_transform_* :312-352) and mixes images with a Python loop of small
+kernels behind four all_gathers (generate_cut_gather_* :354-477).  Here
 
-  * the IMAGE keeps the reference's PIL path (bilinear resize, reflect pad, colour jitter, blur: BASELINE north_star
-    leaves the augmentation of images on the PyTorch/PIL path) -- it is also what draws the random geometry, so the
-    Python / torch / NumPy RNG streams are consumed exactly as the reference consumes them;
+  * the host only DRAWS: `draw_image_params` consumes the Python and torch RNG streams exactly as the reference's PIL
+    chain does (`_augment_image`, kept as the in-tree reference) and returns the geometry and the per-image jitter / blur
+    parameters, without touching pixels;
+  * the IMAGE never leaves the GPU: `css_aug_image` replays Pillow's 8-bit arithmetic (bilinear resize, reflect pad,
+    crop, ColorJitter, GaussianBlur, flip, to_tensor + normalize) bit-identically (`transform_images`);
   * the MAPS never leave the GPU: `css_aug_index` + `css_aug_maps` replay the drawn geometry (Pillow NEAREST resize
     table, bottom/right padding with 255 / 0, crop, flip) and the 8-bit round trip (label -1 <-> 255, conf ->
     floor(conf * 255) / 255) bit-exactly;
@@ -33,7 +34,7 @@ _STD = (0.229, 0.224, 0.225)
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# image side (CPU, PIL) -- also the source of the random geometry
+# image side: the PIL chain (the reference), the host-side draws, the GPU replay
 # ---------------------------------------------------------------------------------------------------------------
 def _tv():
     import torchvision.transforms as T
@@ -76,6 +77,51 @@ def _augment_image(pil, crop_size, scale_size, augmentation):
             flip = True
     img = TF.normalize(TF.to_tensor(pil), mean=list(_MEAN), std=list(_STD))
     return img, (rh, rw, int(top), int(left), int(flip))
+
+
+# Columns of the per-image parameter table (float32 [B, 11]; every value is exactly representable): jitter on/off, the
+# ColorJitter order (0 brightness, 1 contrast, 2 saturation, 3 hue), the three blend factors, the hue shift as the byte
+# torchvision adds to H, blur on/off and the GaussianBlur radius (Pillow takes it as a C float).
+IMAGE_PARAMS = ("jitter", "order0", "order1", "order2", "order3", "brightness", "contrast", "saturation", "hue_byte", "blur",
+                "radius")
+
+
+def draw_image_params(B, H, W, crop_size, scale_size, augmentation):
+    """Draws what `_augment_image` draws for B images of H x W, in the same order from the same generators (`random`,
+    torch's CPU generator; numpy is not used), without touching pixels.  Returns (geometry int32 [B,5] = resized_h,
+    resized_w, top, left, flip -- what `transform_maps` replays -- and the float32 [B, len(IMAGE_PARAMS)] table)."""
+    T, _ = _tv()
+    jitter = T.ColorJitter((0.75, 1.25), (0.75, 1.25), (0.75, 1.25), (-0.25, 0.25))
+    geometry = np.zeros((B, 5), np.int32)
+    params = np.zeros((B, len(IMAGE_PARAMS)), np.float32)
+    for k in range(B):
+        ratio = random.uniform(scale_size[0], scale_size[1])
+        rh, rw = int(H * ratio), int(W * ratio)
+        crop = (W, H) if crop_size == -1 else crop_size
+        ch, cw = int(crop[0]), int(crop[1])
+        # a stand-in of the padded image's shape: RandomCrop draws nothing when it equals the crop
+        top, left, _, _ = T.RandomCrop.get_params(torch.zeros(()).expand(3, max(rh, ch), max(rw, cw)), output_size=(ch, cw))
+        flip = 0
+        if augmentation:
+            if torch.rand(1) > 0.2:
+                order, fb, fc, fs, fh = jitter.get_params(jitter.brightness, jitter.contrast, jitter.saturation, jitter.hue)
+                params[k, 0] = 1
+                params[k, 1:5] = order.numpy()
+                params[k, 5:8] = fb, fc, fs
+                params[k, 8] = np.int32(fh * 255).astype(np.uint8)           # torchvision's adjust_hue byte
+            if torch.rand(1) > 0.5:
+                params[k, 9], params[k, 10] = 1, random.uniform(0.15, 1.15)
+            if torch.rand(1) > 0.5:
+                flip = 1
+        geometry[k] = rh, rw, top, left, flip
+    return geometry, params
+
+
+def image_lut():
+    """float32 [3,256]: byte -> to_tensor + normalize, computed with the very torch CPU ops torchvision applies."""
+    _, TF = _tv()
+    x = torch.arange(256, dtype=torch.uint8).view(1, 1, 256).expand(3, 1, 256).to(torch.float32).div(255)
+    return TF.normalize(x, mean=list(_MEAN), std=list(_STD)).reshape(3, 256).contiguous()
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -144,20 +190,70 @@ def transform_maps(labels, confs, geometry, crop_hw, max_resized=None):
     return out_l, out_c
 
 
+_LUTS = {}
+
+
+def _lut(dev):
+    """image_lut() on `dev`, made once per device (so that a captured CUDA graph finds it in place)."""
+    key = str(dev)
+    if key not in _LUTS:
+        _LUTS[key] = image_lut().to(dev)
+    return _LUTS[key]
+
+
+def _table_arg(t, shape, dtype, dev, name):
+    if isinstance(t, torch.Tensor) and t.is_cuda:
+        if tuple(t.shape) != shape:
+            raise RuntimeError(f"css_b200: `{name}` must be {list(shape)}, got {list(t.shape)}")
+        return t.to(dtype).contiguous(), None
+    a = np.asarray(t.cpu() if isinstance(t, torch.Tensor) else t, dtype={torch.int32: np.int32, torch.float32: np.float32}[dtype])
+    if a.shape != shape:
+        raise RuntimeError(f"css_b200: `{name}` must be {list(shape)}, got {list(a.shape)}")
+    a = np.ascontiguousarray(a)
+    return torch.from_numpy(a).pin_memory().to(dev, non_blocking=True), a
+
+
+def transform_images(images, geometry, params, crop_hw):
+    """The image side of `_augment_image` for a whole batch on the GPU, bit-identical to the Pillow chain.
+    images: unnormalised CUDA float32 [B,3,H,W] in [0, 1] (what `_unnormalise` returns); geometry: int [B,5] and params:
+    float [B, len(IMAGE_PARAMS)] as drawn by `draw_image_params`.  Returns the normalised float32 [B,3,ch,cw].  With
+    CUDA `geometry` and `params` the call does no host synchronisation (CUDA-graph capturable)."""
+    if not isinstance(images, torch.Tensor) or not images.is_cuda:
+        raise RuntimeError("css_b200: `images` must be a CUDA tensor (no CPU fallback)")
+    if images.dtype != torch.float32 or images.dim() != 4 or images.shape[1] != 3:
+        raise RuntimeError(f"css_b200: `images` must be float32 [B,3,H,W], got {images.dtype} {list(images.shape)}")
+    images = images.contiguous()
+    B, _, H, W = images.shape
+    ch, cw = int(crop_hw[0]), int(crop_hw[1])
+    if ch <= 0 or cw <= 0:
+        raise RuntimeError(f"css_b200: bad crop size {(ch, cw)}")
+    dev = images.device
+    geo, _ = _table_arg(geometry, (B, 5), torch.int32, dev, "geometry")
+    par, par_host = _table_arg(params, (B, len(IMAGE_PARAMS)), torch.float32, dev, "params")
+    if par_host is not None:
+        r = par_host[par_host[:, IMAGE_PARAMS.index("blur")] != 0, IMAGE_PARAMS.index("radius")]
+        if ((r < 0) | (r > 4)).any():
+            raise RuntimeError("css_b200: GaussianBlur radius must be in [0, 4]")
+    lib = _lib.load()
+    out = torch.empty((B, 3, ch, cw), device=dev, dtype=torch.float32)
+    ws_bytes = lib.css_aug_image_workspace_bytes(B, ch, cw)
+    ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+    with torch.cuda.device(dev):
+        check(lib.css_aug_image(ptr(images), B, H, W, ptr(geo), ptr(par), ptr(_lut(dev)), ch, cw, ptr(ws), ws_bytes, ptr(out),
+                                stream_ptr()), "css_aug_image")
+    return out
+
+
 def _batch_transform(images, labels, confs, crop_size, scale_size, augmentation):
     if not images.is_cuda:
         raise RuntimeError("css_b200: `images` must be a CUDA tensor (no CPU fallback)")
-    _, TF = _tv()
-    dev = images.device
-    host = _unnormalise(images).cpu()                       # ONE device->host copy for the whole batch
-    out_img, geometry = [], []
-    for k in range(host.shape[0]):
-        img, geo = _augment_image(TF.to_pil_image(host[k]), crop_size, scale_size, augmentation)
-        out_img.append(img)
-        geometry.append(geo)
-    crop_hw = out_img[0].shape[1:]
-    out_l, out_c = transform_maps(labels, confs, np.asarray(geometry, np.int32), crop_hw)
-    image_trans = torch.stack(out_img).pin_memory().to(dev, non_blocking=True)
+    B, _, H, W = images.shape
+    geometry, params = draw_image_params(B, H, W, crop_size, scale_size, augmentation)
+    crop = (W, H) if crop_size == -1 else crop_size
+    crop_hw = (int(crop[0]), int(crop[1]))
+    geo = torch.from_numpy(geometry).pin_memory().to(images.device, non_blocking=True)
+    image_trans = transform_images(_unnormalise(images), geo, params, crop_hw)
+    out_l, out_c = transform_maps(labels, confs, geo, crop_hw, max_resized=int(geometry[:, :2].max()))
     return image_trans, out_l, out_c
 
 

@@ -279,6 +279,32 @@ int css_cut_mix(const float* image, const int64_t* label_a, const int64_t* label
                 float* out_image, int64_t* out_label_a, int64_t* out_label_b, float* out_conf_a, float* out_conf_b,
                 void* stream);
 
+/* ---- the image's trip through the same augmentation, bit-identical to the Pillow chain ----------------------------------------
+ * to_pil_image -> bilinear resize -> reflect pad (bottom / right) -> crop -> ColorJitter -> GaussianBlur -> hflip -> to_tensor +
+ * normalize, in Pillow's 8-bit arithmetic (css_b200/aug.py::_augment_image is the reference; oracle/pil_oracle.py the
+ * specification).  Replaces, for the image, the device->host copy, the per-image PIL loop and the host->device copy of
+ * batch_transform_* (dataset_helpers/VOC.py:126-196, 312-352).
+ *   images   f32[B,3,H,W] unnormalised, in [0, 1] (byte = trunc(x * 255))
+ *   geometry i32[B,5]     resized_h, resized_w, top, left, flip (as for css_aug_maps)
+ *   params   f32[B,CSS_AUG_IMAGE_PARAMS] per image, columns CSS_AUG_P_*: jitter on/off, the four-op order (0 brightness,
+ *            1 contrast, 2 saturation, 3 hue), the three blend factors, the hue shift as a byte added to H, blur on/off and
+ *            the GaussianBlur radius, which must be <= 4 (integer box radius <= 3)
+ *   lut      f32[3,256]  byte -> normalised value per channel (to_tensor + normalize)
+ *   workspace of css_aug_image_workspace_bytes(B, ch, cw) bytes -> out f32[B,3,ch,cw]
+ */
+#define CSS_AUG_IMAGE_PARAMS   11
+#define CSS_AUG_P_JITTER       0
+#define CSS_AUG_P_ORDER        1    /* [4] */
+#define CSS_AUG_P_BRIGHTNESS   5
+#define CSS_AUG_P_CONTRAST     6
+#define CSS_AUG_P_SATURATION   7
+#define CSS_AUG_P_HUE_BYTE     8
+#define CSS_AUG_P_BLUR         9
+#define CSS_AUG_P_RADIUS       10
+size_t css_aug_image_workspace_bytes(int B, int ch, int cw);
+int css_aug_image(const float* images, int B, int H, int W, const int32_t* geometry, const float* params, const float* lut,
+                  int ch, int cw, void* workspace, size_t workspace_bytes, float* out, void* stream);
+
 /* ---- the exchange step over NVLink peer memory (SURVEY.md 8(e)) -----------------------------------------------------------------
  * Sum of every rank's class_stats [C, D+1] block over the ranks of ONE node, in rank order (bit-identical on all ranks).
  * Replaces concat_all_gather of rep / label (loss.py:77,81; ddp_model.py:241-250) and, on one node, the NCCL all-reduce.

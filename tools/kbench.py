@@ -133,8 +133,13 @@ def main():
     cu2 = torch.rand(B, H, W, generator=g0).to(dev)
     res["aug maps trip: index + 3 maps (8(f)-2, not in path sum)"] = timeit(
         lambda i: aug.transform_maps([fused], [cu, cu2], geo_d, (H, W), max_resized=int(1.5 * max(H, W)) + 1), a.iters)
+    x01 = torch.rand(B, 3, H, W, generator=g0).to(dev)
+    g_img = torch.from_numpy(np.concatenate([geo[:, :4], np.ones((B, 1), np.int32)], 1)).to(dev)
+    p_img = torch.tensor([[1, 3, 1, 0, 2, 1.1, 0.9, 1.2, 17, 1, 1.0]] * B, device=dev)
+    res["aug image trip: resize + jitter + blur + flip (not in path sum)"] = timeit(
+        lambda i: aug.transform_images(x01, g_img, p_img, (H, W)), a.iters)
     img = torch.randn(B, 3, H, W, generator=g0).to(dev)
-    boxes = torch.tensor([[H // 4, 3 * H // 4, W // 8, 7 * W // 8]] * B, dtype=torch.int32, device=dev)
+    boxes =torch.tensor([[H // 4, 3 * H // 4, W // 8, 7 * W // 8]] * B, dtype=torch.int32, device=dev)
     o_img, o_l, o_c, o_c2 = torch.empty_like(img), torch.empty_like(lu), torch.empty_like(cu), torch.empty_like(cu)
 
     def cutmix(i):
