@@ -51,7 +51,11 @@ SIGNATURES = {
     "css_atl_blocks": (c_int, [c_int, c_int]),
     "css_atl_forward": (c_int, [P, P, P, c_float, c_int, c_int, c_int, c_int, P, P, P, P, P, P]),
     "css_atl_backward": (c_int, [P, P, P, P, P, c_int, c_int, c_int, c_int, P, P]),
-    "css_comm_bytes": (ctypes.c_size_t, [c_int]),
+    "css_ohem_workspace_bytes": (ctypes.c_size_t, [c_int, c_int, c_int]),
+    "css_ohem_forward": (c_int, [P, P, P, ctypes.c_longlong, c_float, c_int, c_int, c_int, c_int, c_int, P, ctypes.c_size_t, P, P, P,
+                                 P]),
+    "css_ohem_backward": (c_int, [P, P, P, P, c_int, c_int, c_int, c_int, P, ctypes.c_size_t, P, P]),
+    "css_comm_bytes":(ctypes.c_size_t, [c_int]),
     "css_comm_alloc": (c_int, [c_int, ctypes.POINTER(ctypes.c_void_p)]),
     "css_comm_free": (c_int, [P]),
     "css_comm_set_timeout_ms": (c_int, [ctypes.c_ulonglong]),

@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcss_b200.so")
-SOURCES = ["css_api.cu", "css_sim.cu", "css_sim_tc.cu", "css_select.cu", "css_stream.cu", "css_proto.cu", "css_score.cu", "css_grad.cu", "css_atl.cu", "css_aug.cu", "css_aug_image.cu", "css_comm.cu"]
+SOURCES = ["css_api.cu", "css_sim.cu", "css_sim_tc.cu", "css_select.cu", "css_stream.cu", "css_proto.cu", "css_score.cu", "css_grad.cu", "css_atl.cu", "css_ohem.cu", "css_aug.cu", "css_aug_image.cu", "css_comm.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--use_fast_math=false"]
 
 

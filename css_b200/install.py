@@ -3,7 +3,7 @@
     import css_b200.install; css_b200.install.install()      # BEFORE importing ori_pseudo / mix_label / cross_label
 
 The three scripts bind their names with `from ... import` at import time (mix_label.py:12,21), so the reference modules
-are patched first: `generalframeworks.loss.loss.Contrast_Loss` and `generalframeworks.networks.ddp_model.Model_*` are
+are patched first: `generalframeworks.loss.loss.Contrast_Loss` (and the two logit-space losses) and `generalframeworks.networks.ddp_model.Model_*` are
 replaced by the css_b200 classes, whose hooks are pointed at the reference's own network and augmentation functions.
 """
 import importlib
@@ -40,6 +40,7 @@ def install(reference_root=None, stub_shutup=True, gpu_aug=False):
             setattr(h, name, getattr(_aug, name))
     ref_loss.Contrast_Loss = _loss.Contrast_Loss
     ref_loss.Attention_Threshold_Loss = _loss.Attention_Threshold_Loss
+    ref_loss.ProbOhemCrossEntropy2d = _loss.ProbOhemCrossEntropy2d
     ref_model.Model_ori_pseudo = _models.Model_ori_pseudo
     ref_model.Model_mix = _models.Model_mix
     ref_model.Model_cross = _models.Model_cross

@@ -339,3 +339,95 @@ class Attention_Threshold_Loss(nn.Module):
         with torch.cuda.device(pred.device):
             return _AttentionThresholdFn.apply(pred_c, pseudo_label.long().contiguous(), logits.float().contiguous(),
                                                self.strong_threshold)
+
+
+# the 19 CityScapes class weights of the reference (loss.py:8-46, use_weight=True)
+CITYSCAPES_CLASS_WEIGHTS = (0.8373, 0.918, 0.866, 1.0345, 1.0166, 0.9969, 0.9754, 1.0489, 0.8786, 1.0023,
+                            0.9539, 0.9843, 1.1116, 0.9037, 1.0865, 1.0955, 1.0865, 1.1529, 1.0507)
+_INT32_MAX = 2 ** 31 - 1
+
+
+class _OhemFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, pred, target, weight, ignore_index, thresh, min_kept, ws, threshold, counts):
+        lib = _lib.load()
+        B, C, H, W = pred.shape
+        loss = torch.empty((), device=pred.device, dtype=torch.float32)
+        check(lib.css_ohem_forward(ptr(pred), ptr(target), ptr(weight), int(ignore_index), float(thresh), int(min_kept), B, C, H, W,
+                                   ptr(ws), ws.numel(), ptr(loss), ptr(threshold), ptr(counts), stream_ptr()), "css_ohem_forward")
+        ctx.save_for_backward(pred, target, weight, ws)
+        return loss
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        pred, target, weight, ws = ctx.saved_tensors
+        lib = _lib.load()
+        B, C, H, W = pred.shape
+        grad_pred = torch.empty_like(pred)
+        go = grad_out.detach().to(torch.float32).contiguous()
+        with torch.cuda.device(pred.device):
+            check(lib.css_ohem_backward(ptr(go), ptr(pred), ptr(target), ptr(weight), B, C, H, W, ptr(ws), ws.numel(), ptr(grad_pred),
+                                        stream_ptr()), "css_ohem_backward")
+        return grad_pred, None, None, None, None, None, None, None, None
+
+
+class ProbOhemCrossEntropy2d(nn.Module):
+    """Drop-in for generalframeworks/loss/loss.py:8-46 (same constructor and forward): the supervised OHEM cross-entropy.
+
+    Pixels whose label is not `ignore_index` are valid.  With p_t the softmax probability of a pixel's own label, the loss is
+    the (class-weighted) mean cross-entropy over the valid pixels with p_t <= T, T = max(float32(thresh), the min_kept-th
+    smallest p_t); over all valid pixels when min_kept <= 0 or fewer than min_kept pixels are valid; nan when none is valid.
+    One fused pass over `pred` forward (plus, only when the threshold is not float32(thresh), an exact radix select over the
+    per-pixel p_t) and one backward, all on the device with no host synchronisation: it can be captured in a CUDA graph.
+
+    Differences from the reference:
+      * the reference's `logger.info('Labels: ...')` when min_kept > #valid is dropped (it needs the count on the host);
+      * labels outside [0, C) other than ignore_index are treated as ignored (torch would raise a device-side assert);
+      * only reduction='mean' exists (what the scripts use); `down_ratio` is accepted and unused, as in the reference;
+      * `pred` must be a float32 CUDA tensor (no CPU fallback); the caller's `target` is never modified.
+    After each forward, `self.last` holds device tensors `num_valid`, `threshold` (the T used, +inf when OHEM did not apply),
+    `num_kept` and `p_t` ([B,H,W], nan on ignored pixels; kept = p_t <= threshold), for verification; nothing reads them on
+    the training path.
+    """
+
+    def __init__(self, ignore_index, reduction='mean', thresh=0.6, min_kept=256, down_ratio=1, use_weight=False):
+        super().__init__()
+        if reduction != 'mean':
+            raise ValueError(f"css_b200: ProbOhemCrossEntropy2d supports reduction='mean' only, got {reduction!r}")
+        self.ignore_index = ignore_index
+        self.reduction = reduction
+        self.thresh = float(thresh)
+        self.min_kept = int(min_kept)
+        self.down_ratio = down_ratio
+        self.use_weight = use_weight
+        self.register_buffer("weight", torch.tensor(CITYSCAPES_CLASS_WEIGHTS, dtype=torch.float32) if use_weight else None)
+        self.last = None
+
+    def forward(self, pred, target):
+        if not (pred.is_cuda and target.is_cuda):
+            raise RuntimeError("css_b200: ProbOhemCrossEntropy2d needs CUDA tensors (no CPU fallback)")
+        if pred.dtype != torch.float32:
+            raise RuntimeError(f"css_b200: pred must be float32, got {pred.dtype}")
+        if pred.dim() != 4 or target.numel() != pred.shape[0] * pred.shape[2] * pred.shape[3]:
+            raise RuntimeError("css_b200: pred must be [B,C,H,W] and target hold B*H*W labels")
+        if target.dtype.is_floating_point or target.dtype == torch.bool:
+            raise RuntimeError(f"css_b200: target must hold integer labels, got {target.dtype}")
+        weight = None
+        if self.weight is not None:
+            if self.weight.numel() != pred.shape[1]:
+                raise RuntimeError(f"css_b200: use_weight=True has {self.weight.numel()} class weights, pred has {pred.shape[1]} classes")
+            weight = self.weight if self.weight.device == pred.device else self.weight.to(pred.device)
+        pred_c = pred.contiguous()                           # channels-last or strided pred: one copy into NCHW
+        target_c = target.reshape(-1).to(torch.int64).contiguous()
+        B, _, H, W = pred.shape
+        dev = pred.device
+        # per-call scratch (the forward writes it, the backward reads lse / p_t / T from it); p_t per pixel comes first
+        ws = torch.empty(_lib.load().css_ohem_workspace_bytes(B, H, W), device=dev, dtype=torch.uint8)
+        threshold = torch.empty((), device=dev, dtype=torch.float32)
+        counts = torch.empty(2, device=dev, dtype=torch.int32)
+        min_kept = min(self.min_kept, _INT32_MAX)            # beyond any int32 pixel count: OHEM never applies either way
+        with torch.cuda.device(dev):
+            loss = _OhemFn.apply(pred_c, target_c, weight, int(self.ignore_index), self.thresh, min_kept, ws, threshold, counts)
+        self.last = dict(num_valid=counts[0], threshold=threshold, num_kept=counts[1],
+                         p_t=ws[:4 * B * H * W].view(torch.float32).view(B, H, W))
+        return loss

@@ -245,6 +245,25 @@ int css_atl_forward(const float* pred, const int64_t* label, const float* conf, 
 int css_atl_backward(const float* grad_out, const float* pred, const int64_t* label, const float* lse, const float* scale,
                      int B, int C, int H, int W, float* grad_pred, void* stream);
 
+/* ---- ProbOhemCrossEntropy2d, the supervised OHEM cross-entropy (DESIGN.md f-5) ---------------------------------------------------
+ * valid = target != ignore_index (labels outside [0,C) are treated as ignored); p_t = softmax(pred[:,p])[target_p].
+ * When min_kept > 0 and #valid >= min_kept: kept = valid & p_t <= T, T = max(thresh, kth), kth = the min_kept-th smallest p_t
+ * of the valid pixels, found by an exact radix select on the device; otherwise kept = valid and T = +inf.  All comparisons are
+ * float32.  loss = sum_kept w[y] (lse - x_y) / sum_kept w[y], nan when nothing is kept.  Replaces loss.py:8-46 (forward) and
+ * its autograd backward; unlike the reference it makes no host synchronisation and is CUDA-graph capturable.
+ *   pred [B,C,H,W] f32, target [B,H,W] i64, weight f32[C] or NULL (= all ones)
+ *   workspace of css_ohem_workspace_bytes(B,H,W) bytes (0 for a bad size); the forward writes it and the backward reads it.
+ *   After the forward its first B*H*W floats hold p_t per pixel id (NaN on ignored pixels): kept = p_t <= threshold.
+ *   loss f32[1], threshold f32[1] = T, counts i32[2] = #valid, #kept
+ *   backward: grad_pred [B,C,H,W] f32 = grad_out * w[y] / sum_kept w * (softmax - onehot) on kept pixels, 0 elsewhere
+ */
+size_t css_ohem_workspace_bytes(int B, int H, int W);
+int css_ohem_forward(const float* pred, const int64_t* target, const float* weight, long long ignore_index, float thresh,
+                     int min_kept, int B, int C, int H, int W, void* workspace, size_t workspace_bytes, float* loss,
+                     float* threshold, int32_t* counts, void* stream);
+int css_ohem_backward(const float* grad_out, const float* pred, const int64_t* target, const float* weight, int B, int C, int H,
+                      int W, const void* workspace, size_t workspace_bytes, float* grad_pred, void* stream);
+
 /* ---- augmentation hand-off of the label / confidence maps (SURVEY.md 8(f)-2) ------------------------------------------------
  * The maps' trip tensor -> PIL 'L' image -> NEAREST resize -> bottom/right pad (255 / 0) -> crop -> hflip -> tensor, kept on the
  * GPU.  Replaces, for the maps, tensor_to_pil_* + transform_* + the host->device copies of batch_transform_*

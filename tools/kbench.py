@@ -119,6 +119,13 @@ def main():
         (gr,) = torch.autograd.grad(atl(pp_, lu, cu), pp_)
 
     res["attention_threshold_loss fwd+bwd (8(f)-3, not in path sum)"] = timeit(atl_step, a.iters)
+    ohem = css_b200.ProbOhemCrossEntropy2d(ignore_index=-1, thresh=0.7, min_kept=50000 * B).cuda()
+
+    def ohem_step(i):
+        pp_ = pl.detach().requires_grad_(True)
+        (gr,) = torch.autograd.grad(ohem(pp_, lu), pp_)
+
+    res["prob_ohem_ce fwd+bwd (f-5, not in path sum)"] = timeit(ohem_step, a.iters)
     # 8(f)-2: both trips of the maps through the augmentation + CutMix, at the crop size
     from css_b200 import aug
     import numpy as np
