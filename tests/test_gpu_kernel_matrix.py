@@ -8,7 +8,9 @@ into libcss_b200.so.  The declarations below build without a GPU; the tests need
 
 Tolerances are those of DESIGN.md section 2, measured against float64: similarities / probabilities abs 1e-6, norms rel 1e-6,
 confidences abs 2e-6, losses and gradients rel 1e-4 (gradient elements with 2e-5 of the largest element as absolute slack,
-as in test_gpu_fullsize.py).  Set CSS_B200_F64_REPORT=<file> to write the largest error of each kernel family as JSON.
+as in test_gpu_fullsize.py).  At the models' temperatures (0.25, 0.1) a probability or confidence bound is the larger of
+these and the error of torch's own float32 statements on the same inputs (f32_bound).  Set CSS_B200_F64_REPORT=<file> to
+write the largest error of each kernel family as JSON.
 """
 import json
 import math
@@ -18,6 +20,7 @@ import re
 import numpy as np
 import pytest
 import torch
+import torch.nn.functional as F
 
 from tests.helpers import TAU
 
@@ -76,6 +79,10 @@ REP_CASES = _rep_cases()
 UPSAMPLE_CASES = [
     pytest.param(21, 41, 41, 161, 161, 0.5, "staged", "upsample_label_fuse_kernel<true, 21>", id="C21-staged"),
     pytest.param(19, 49, 33, 193, 129, 0.3, "staged", "upsample_label_fuse_kernel<true, 19>", id="C19-staged"),
+    pytest.param(21, 41, 41, 161, 161, 0.25, "staged", "upsample_label_fuse_kernel<true, 21>", id="C21-staged-t0.25"),
+    pytest.param(21, 41, 41, 161, 161, 0.1, "staged", "upsample_label_fuse_kernel<true, 21>", id="C21-staged-t0.1"),
+    pytest.param(19, 49, 33, 193, 129, 0.25, "staged", "upsample_label_fuse_kernel<true, 19>", id="C19-staged-t0.25"),
+    pytest.param(19, 49, 33, 193, 129, 0.1, "staged", "upsample_label_fuse_kernel<true, 19>", id="C19-staged-t0.1"),
     pytest.param(7, 33, 31, 129, 121, 0.5, "staged", "upsample_label_fuse_kernel<true, 0>", id="C7-staged"),
     pytest.param(32, 20, 21, 77, 81, 0.7, "staged", "upsample_label_fuse_kernel<true, 0>", id="C32-staged"),
     pytest.param(21, 40, 50, 40, 50, 0.5, "optin", "upsample_label_fuse_kernel<true, 21>", id="C21-optin"),
@@ -142,16 +149,59 @@ def peer_kernel(world):
 
 PEER_KERNELS = [peer_kernel(w) for w in PEER_WORLDS]
 
+# the models' own temperatures: Model_mix 0.25, Model_cross 0.1 (models.py:93,116); an error in a cosine reaches their
+# probabilities scaled by 1/temp
+MODEL_TEMPS = (0.25, 0.1)
+REP_TEMP_CASES = [pytest.param(C, t, ["proto_prep_kernel", rep_kernel((C + 3) // 4, True, F32, C == 21)], id=f"C{C}-t{t}")
+                  for C in REP_CLASSES for t in MODEL_TEMPS]
+SIM_MODES = ((None, "cos"), (0.5, "t0.5"), (0.25, "t0.25"), (0.1, "t0.1"))     # (softmax temperature or None = cosine, id)
+
+# channels-last rep pass (css_sim_tc.cu rep_pass_nhwc_kernel<NP>: NP = 3 for C <= 24, 4 above, with padded class columns)
+NHWC_CLASSES = (1, 5, 19, 21, 24, 25, 31, 32)
+NHWC_SHAPES = ("one_tile", "exact128", "ragged", "sub_wave", "city193")
+
+
+def nhwc_kernel(C):
+    return f"rep_pass_nhwc_kernel<{3 if C <= 24 else 4}>"
+
+
+NHWC_CASES = [pytest.param(C, shape, t, ["proto_prep_tc_kernel", nhwc_kernel(C)], id=f"C{C}-{shape}-{tid}")
+              for C in NHWC_CLASSES for shape in NHWC_SHAPES for t, tid in SIM_MODES]
+NHWC_ALIGN_CASES = [pytest.param(4, ["proto_prep_tc_kernel", nhwc_kernel(21)], id="offset16B-channels_last"),
+                    pytest.param(1, ["proto_prep_kernel", rep_kernel(6, True, F32, True)], id="offset4B-nchw_copy")]
+NHWC_REFRESH_KERNELS = ["rows_verify_rm_kernel", nhwc_kernel(1)]
+NHWC_LOSS_KERNELS = ["rows_verify_rm_kernel", nhwc_kernel(1), "grad_rows_kernel"]
+
+# NCHW tensor-core rep pass (css_sim_tc.cu rep_pass_tc_kernel<ROWS, NP>, opt-in with css_set_rep_pass_path(1)); the map at a
+# storage offset of 0..3 floats: 1..3 put every plane window's start off 16 bytes (the base16 lead-in) and send the first
+# plane through the loader's per-lane copy
+TC_CLASSES = (1, 5, 21, 24, 25, 32)
+TC_SHAPES = {"hw63": (1, 7, 9), "hw128": (2, 8, 16), "hw129": (3, 3, 43), "hw510": (2, 17, 30), "city193": (8, 193, 193)}
+TC_OFFSETS = (0, 1, 2, 3)
+
+
+def tc_kernels(C, rows):
+    return ["proto_prep_tc_kernel", f"rep_pass_tc_kernel<{_b(rows)}, {3 if C <= 24 else 4}>"]
+
+
+TC_CASES = ([pytest.param(C, "hw510", off, t, tc_kernels(C, t is not None), id=f"C{C}-hw510-off{off}-{tid}")
+             for C in TC_CLASSES for off in TC_OFFSETS for t, tid in SIM_MODES]
+            + [pytest.param(C, shape, off, t, tc_kernels(C, t is not None), id=f"C{C}-{shape}-off{off}-{tid}")
+               for shape in ("hw63", "hw128", "hw129", "city193") for off in TC_OFFSETS for C, t, tid in ((21, 0.1, "t0.1"), (25, None, "cos"))])
+
 
 def declared_kernels():
     """Every instantiation some case of this module asserts it launches."""
     out = set()
-    for cases in (REP_CASES, SCORER_CASES, NN_EDGE_CASES, TEMP_SWITCH_CASES, BENCH_CASES, ATL_CASES):
+    for cases in (REP_CASES, REP_TEMP_CASES, SCORER_CASES, NN_EDGE_CASES, TEMP_SWITCH_CASES, BENCH_CASES, ATL_CASES, NHWC_CASES,
+                  NHWC_ALIGN_CASES, TC_CASES):
         for p in cases:
             out.update(p.values[-1])
     out.update(p.values[-1] for p in UPSAMPLE_CASES)
     out.update(ROWS_VERIFY_KERNELS)
     out.update(PEER_KERNELS)
+    out.update(NHWC_REFRESH_KERNELS)
+    out.update(NHWC_LOSS_KERNELS)
     out.add(scorer_kernel("grad-f32-reg", False, False))           # test_scorer_anti_aligned_candidates (online-max side)
     out.add(scorer_kernel("grad-f32-reg", True, False))
     return out
@@ -235,6 +285,74 @@ def check_loss(got, ref, rtol=RTOL, family=None):
         record(family + " loss (rel)", err)
 
 
+def f32_bound(bound, torch_f32_err, family):
+    """At the models' temperatures the bound on a probability or confidence is the larger of the fixed one and the error of
+    torch's own float32 statements on the same inputs, measured against the same float64 reference (DESIGN.md section 2)."""
+    record(family, torch_f32_err)
+    return max(bound, torch_f32_err)
+
+
+def torch_f32_prob(x, protos, temp):
+    """ddp_model.py:147-154 as the reference runs it in float32: F.normalize, mm (no TF32), softmax."""
+    B, D, h, w = x.shape
+    prev = torch.backends.cuda.matmul.allow_tf32
+    torch.backends.cuda.matmul.allow_tf32 = False
+    try:
+        sim = F.normalize(x.float().permute(0, 2, 3, 1).reshape(-1, D), dim=-1) @ F.normalize(protos.float(), dim=-1).T
+    finally:
+        torch.backends.cuda.matmul.allow_tf32 = prev
+    return torch.softmax(sim / temp, dim=1).reshape(B, h, w, -1).permute(0, 3, 1, 2)
+
+
+def check_sim_map(out, x, protos, temp, family):
+    """A cosine map (temp None) or softmax(cos / temp) against float64: abs 1e-6 (at the models' temperatures, see f32_bound).
+    x carries rich_map's content: a zero prototype row and a zero-norm pixel give exact zeros in a cosine map."""
+    from oracle import f64_ref as R
+    C = protos.shape[0]
+    if temp is None:
+        err = (out.double() - R.cos_sim_map(x, protos)).abs().max().item()
+        record(family + " sim", err)
+        assert err <= 1e-6, f"cos: max abs error {err:.3e} vs float64"
+        if C > 1:
+            assert (out[:, C // 2] == 0).all(), "the zero prototype row has a non-zero similarity"
+        assert (out[0, :, 0, 1] == 0).all(), "the zero-norm pixel has a non-zero similarity"
+        return
+    ref = R.proto_softmax_sim(x, protos, temp)
+    err = (out.double() - ref).abs().max().item()
+    bound = 1e-6
+    if temp in MODEL_TEMPS:
+        bound = f32_bound(bound, (torch_f32_prob(x, protos, temp).double() - ref).abs().max().item(), f"torch float32 prob t{temp}")
+    record(f"{family} prob t{temp}" if temp in MODEL_TEMPS else family + " prob", err)
+    assert err <= bound, f"softmax t{temp}: max abs error {err:.3e} vs float64 (bound {bound:.3e})"
+
+
+def check_norms(norms, x, family):
+    nref = torch.linalg.vector_norm(x.double(), dim=1).reshape(-1)
+    assert norms[1].item() == 0.0                                      # rich_map's zero-norm pixel (0, 0, 1)
+    rel = ((norms.double() - nref).abs() / nref.clamp_min(1e-300)).max().item()
+    record(family + " norms (rel)", rel)
+    assert rel <= 1e-6, f"norms: max rel error {rel:.3e} vs float64"
+
+
+def rich_map(B, h, w, C, seed):
+    """A [B,256,h,w] map and [C,256] prototypes on the GPU with the content where a similarity kernel can go wrong: a zero-norm
+    pixel, a zero prototype row (C > 1), a pixel that is a multiple of the last prototype (cos = 1), a pixel with one channel
+    ~1e3 and the rest ~1e-3.  Normal values nearly always have some of their low 13 mantissa bits set, the bits a TF32 operand
+    drops, so the lo term of the tensor-core kernels' hi/lo split carries weight."""
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    x = torch.randn(B, 256, h, w, generator=g, device="cuda")
+    assert ((x.view(torch.int32) & 0x1FFF) != 0).float().mean().item() > 0.99
+    protos = 0.5 * torch.randn(C, 256, generator=g, device="cuda")
+    if C > 1:
+        protos[C // 2] = 0
+    px = x.view(B, 256, h * w)
+    px[0, :, 1] = 0
+    px[0, :, 2] = 3 * protos[C - 1]
+    px[0, :, 3] *= 1e-3
+    px[0, 7, 3] = 1000.123
+    return x, protos
+
+
 # ---------------------------------------------------------------------------------------------------------------------------
 # rep pass (css_sim.cu rep_pass_kernel: NG 1..8 x ROWS x fp32 / bf16, the rows-only pass)
 # ---------------------------------------------------------------------------------------------------------------------------
@@ -306,6 +424,17 @@ def _run_pair(run, rep, dtype):
     return first, second
 
 
+@pytest.mark.parametrize("C,temp,kernels", REP_TEMP_CASES)
+def test_rep_pass_model_temps(lib, C, temp, kernels):
+    """The shipped fp32 student pass at the temperatures the models run it at."""
+    import css_b200
+    B, h, w = rep_shape("ragged")
+    x, protos = rich_map(B, h, w, C, seed=3000 + 10 * C + int(1 / temp))
+    prob, names = launched(lambda: css_b200.ops.proto_softmax_sim(x, protos, temp))
+    assert_launched(kernels, names)
+    check_sim_map(prob, x, protos, temp, "rep_pass")
+
+
 # ---------------------------------------------------------------------------------------------------------------------------
 # fused up-sample + softmax + max + fusion (css_sim.cu upsample_label_fuse_kernel)
 # ---------------------------------------------------------------------------------------------------------------------------
@@ -334,8 +463,12 @@ def test_upsample_label_fuse(C, h, w, H, W, temp, tile, kernel):
     for key, src, t in (("rep", sim, temp), ("cls", logits, None)):
         conf, label, margin = R.upsample_softmax_max(src, (H, W), t)
         err = (o["conf_" + key].double() - conf).abs().max().item()
-        record("upsample conf", err)
-        assert err <= 2e-6, f"conf_{key}: max abs error {err:.3e} vs float64"
+        bound = 2e-6
+        if t in MODEL_TEMPS:
+            f32 = torch.softmax(F.interpolate(src, size=(H, W), mode="bilinear", align_corners=True) / t, dim=1).max(dim=1).values
+            bound = f32_bound(bound, (f32.double() - conf).abs().max().item(), f"torch float32 upsample conf t{t}")
+        record(f"upsample conf t{t}" if t in MODEL_TEMPS else "upsample conf", err)
+        assert err <= bound, f"conf_{key}: max abs error {err:.3e} vs float64 (bound {bound:.3e})"
         bad = o["label_" + key] != label
         assert not (bad & (margin >= TAU)).any(), f"label_{key} differs away from near-ties"
     fused = torch.where(o["label_rep"] == o["label_cls"], o["label_cls"].float(), torch.full_like(o["fused"], 255.0))
@@ -548,6 +681,224 @@ def test_rows_verify_bf16(lib):
     assert torch.equal(last["rows"], other.permute(0, 2, 3, 1).reshape(-1, 256))
     l_ref, last_ref = run(other, prob.clone())
     assert last_ref["rows_cache_mode"] == "miss" and l_other == l_ref
+
+
+# ---------------------------------------------------------------------------------------------------------------------------
+# channels-last maps (css_sim_tc.cu rep_pass_nhwc_kernel, rows_verify_rm_kernel; css_grad.cu grad_rows_kernel)
+# ---------------------------------------------------------------------------------------------------------------------------
+def nhwc_shape(shape):
+    if shape == "one_tile":
+        return 1, 9, 11                       # N = 99: one partial tile, rows past N zero-filled by the TMA
+    if shape == "exact128":
+        return 4, 8, 12                       # N = 384 = 3 x 128, tiles straddle image boundaries (h*w = 96)
+    if shape == "ragged":
+        return 3, 17, 29                      # N = 1479: partial last tile, straddling tiles
+    if shape == "sub_wave":                   # one tile per CTA on all but a couple of SMs
+        sms = torch.cuda.get_device_properties(0).multi_processor_count
+        h, w = 96, (sms - 2) * 128 // (2 * 96)
+        assert math.ceil(2 * h * w / 128) < sms
+        return 2, h, w
+    return 8, 193, 193                        # city193: ~16 tiles per CTA, every ring and both TMEM buffers wrap their parity
+
+
+def to_channels_last(x):
+    return x.contiguous(memory_format=torch.channels_last)
+
+
+@pytest.mark.parametrize("C,shape,temp,kernels", NHWC_CASES)
+def test_nhwc_rep_pass(lib, C, shape, temp, kernels):
+    """ops.cos_sim_map / proto_softmax_sim on a torch.channels_last map, on both sides of the C <= 24 switch (C 25..31 leave
+    padded class columns in the accumulators, which must not reach a softmax)."""
+    import css_b200
+    B, h, w = nhwc_shape(shape)
+    x, protos = rich_map(B, h, w, C, seed=5000 + 100 * C + h)
+    rep = to_channels_last(x)
+    assert css_b200.ops.is_channels_last(rep)
+    if temp is None:
+        out, names = launched(lambda: css_b200.ops.cos_sim_map(rep, protos))
+    else:
+        out, names = launched(lambda: css_b200.ops.proto_softmax_sim(rep, protos, temp))
+    assert_launched(kernels, names)
+    check_sim_map(out, rep, protos, temp, "nhwc")
+    if temp is not None:
+        cache = out._css_rows
+        assert cache.rows.data_ptr() == rep.data_ptr()                  # the map is its own row table
+        check_norms(cache.norms, rep, "nhwc")
+
+
+@pytest.mark.parametrize("offset,kernels", NHWC_ALIGN_CASES)
+def test_nhwc_alignment(lib, offset, kernels):
+    """A channels-last map at 4 floats into a buffer (16-byte, not 1 KB aligned) is read by the TMA kernel as it is; at 1 float
+    is_channels_last refuses it and the pass runs on the contiguous NCHW copy."""
+    import css_b200
+    B, C, h, w = 2, 21, 13, 11
+    x, protos = rich_map(B, h, w, C, seed=77 + offset)
+    buf = torch.full((x.numel() + 4,), float("nan"), device="cuda")
+    rep = buf.as_strided(x.shape, (h * w * 256, 1, w * 256, 256), offset)
+    rep.copy_(x)
+    assert rep.data_ptr() % 16 == 4 * offset % 16 and rep.data_ptr() % 1024 != 0
+    assert css_b200.ops.is_channels_last(rep) == (offset == 4)
+    prob, names = launched(lambda: css_b200.ops.proto_softmax_sim(rep, protos, 0.5))
+    assert_launched(kernels, names)
+    if offset != 4:
+        assert not {n for n in names if n.startswith("rep_pass_nhwc_kernel")}
+    check_sim_map(prob, x, protos, 0.5, "nhwc")
+    rows = prob._css_rows.rows
+    assert torch.equal(rows, x.permute(0, 2, 3, 1).reshape(-1, 256))
+    assert (rows.data_ptr() == rep.data_ptr()) == (offset == 4)
+    check_norms(prob._css_rows.norms, x, "nhwc")
+
+
+def test_nhwc_norms_and_rows_check(lib):
+    """The norms-only pass (css_rep_pass_nhwc without prototypes) and css_rows_refresh_nhwc: an intact clone leaves the flag at 0
+    and the norms untouched (the pass returns at its guard); a clone that differs in one sampled channel of the last pixel,
+    ((p * 37) & 63) + 64 i (css_sim_tc.cu rows_verify_rm_kernel), raises the flag and has its norms rewritten."""
+    import css_b200
+    from css_b200 import _lib
+    from css_b200._lib import check, ptr, stream_ptr
+    B, h, w = 3, 17, 29
+    N = B * h * w
+    x, _ = rich_map(B, h, w, 1, seed=91)
+    rep = to_channels_last(x)
+    norms, names = launched(lambda: css_b200.ops.rep_norms_nhwc(rep))
+    assert_launched([nhwc_kernel(1)], names)
+    check_norms(norms, x, "nhwc")
+    scratch = torch.empty(2 * 256 * 32, device="cuda")
+
+    def refresh(clone, out):
+        meta = torch.zeros(_lib.META_WORDS, device="cuda", dtype=torch.int32)
+        check(lib.css_rows_refresh_nhwc(ptr(clone), ptr(rep), ptr(out), ptr(scratch), ptr(meta), B, 256, h, w, stream_ptr()),
+              "css_rows_refresh_nhwc")
+        return int(meta[_lib.META_ROWS_STALE].item())
+
+    clone = rep.clone()
+    assert clone.stride() == rep.stride() and clone.data_ptr() != rep.data_ptr()
+    sentinel = torch.full((N,), -7.0, device="cuda")
+    flag, names = launched(lambda: refresh(clone, sentinel))
+    assert_launched(NHWC_REFRESH_KERNELS, names)
+    assert flag == 0 and (sentinel == -7.0).all()
+    p = N - 1
+    for i in range(4):
+        other = rep.clone()
+        css_b200.ops.rows_view(other)[p, ((p * 37) & 63) + 64 * i] += 0.5
+        out = torch.full((N,), -7.0, device="cuda")
+        assert refresh(other, out) == 1, f"a change in sampled channel {((p * 37) & 63) + 64 * i} of pixel {p} went unnoticed"
+        check_norms(out, other, "nhwc")
+
+
+def grad_anchors(spread, N, n, rng):
+    if spread == "uniform":
+        return rng.integers(0, N, n)
+    if spread == "dups":                      # seven distinct pixels hit ~150 times each, 30 % of the slots without an anchor
+        px = rng.choice(rng.integers(0, N, 7), n)
+        px[rng.random(n) < 0.3] = -1
+        return px
+    px = rng.integers(0, N, n)                # "hot": the last pixel hit 600 times among uniform anchors
+    px[rng.choice(n, 600, replace=False)] = N - 1
+    return px
+
+
+GRAD_NHWC_CASES = {"dups_and_absent": (3, 10, 12, 1501, "dups"), "hot_pixel": (2, 21, 23, 2005, "hot"),
+                   "uniform": (4, 81, 81, 2003, "uniform"), "over_32k_anchors": (2, 16, 16, 33003, "uniform")}
+
+
+@pytest.mark.parametrize("name", list(GRAD_NHWC_CASES))
+def test_nhwc_grad_scatter(lib, name):
+    """css_grad_scatter_nhwc against a float64 scatter-add.  n_anchor is never a multiple of the 8 anchors of a CTA.  The output
+    is NaN-filled with guard elements on both sides that must stay NaN.  fp32 atomics add in any order: an element with k
+    contributions t_i is bounded by gamma_(k+1) sum |t_i|, gamma_m = m u / (1 - m u), u = 2^-24 (one rounding per product)."""
+    from css_b200._lib import check, ptr, stream_ptr
+    B2, h, w, n, spread = GRAD_NHWC_CASES[name]
+    N = B2 * h * w
+    rng = np.random.default_rng(n)
+    px = torch.from_numpy(grad_anchors(spread, N, n, rng).astype(np.int32)).cuda()
+    ga = torch.from_numpy(rng.standard_normal((n, 256)).astype(np.float32)).cuda()
+    go = torch.full((), 0.37, device="cuda")
+    G = 4
+    buf = torch.full((N * 256 + 2 * G,), float("nan"), device="cuda")
+    out = buf[G:G + N * 256]
+
+    def run():
+        check(lib.css_grad_scatter_nhwc(ptr(go), ptr(px), ptr(ga), n, B2, 256, h, w, ptr(out), stream_ptr()), "css_grad_scatter_nhwc")
+    _, names = launched(run)
+    assert_launched(["grad_rows_kernel"], names)
+    assert torch.isnan(buf[:G]).all() and torch.isnan(buf[G + N * 256:]).all(), "written outside the gradient"
+    keep = px >= 0
+    terms = go.double() * ga[keep].double()
+    ref = torch.zeros(N, 256, dtype=torch.float64, device="cuda").index_add_(0, px[keep].long(), terms)
+    mag = torch.zeros_like(ref).index_add_(0, px[keep].long(), terms.abs())
+    k = torch.bincount(px[keep].long(), minlength=N).double()[:, None] + 1
+    u = 2.0 ** -24
+    bound = k * u / (1 - k * u) * mag
+    got = out.view(N, 256).double()
+    assert torch.isfinite(got).all()
+    assert torch.equal(got != 0, ref != 0), "the gradient's support is not the anchor pixels"
+    err = (got - ref).abs()
+    record("nhwc grad scatter: max |err| / rigorous bound", (err / bound.clamp_min(1e-300)).max())
+    assert (err <= bound).all(), f"max excess {(err - bound).max().item():.3e}"
+    if spread == "hot":
+        assert int(k[N - 1]) > 600
+
+
+@pytest.mark.parametrize("temp", [0.5, 0.02])
+def test_nhwc_contrast_loss(lib, temp):
+    """Contrast_Loss on a channels-last map handed over as DDP's clone (rows check on the device), with fed draws: loss,
+    gradient and prototypes against float64; the gradient keeps the map's channels-last strides."""
+    import css_b200
+    B2, C, h, w, Q, Nn, seed = 2, 7, 19, 23, 12, 100, 31
+    rep0, label, mask, _, protos = scorer_inputs(B2, C, h, w, seed)
+    rep0 = to_channels_last(rep0)
+    prob = css_b200.ops.proto_softmax_sim(rep0, protos, 0.5)
+    kw = dict(num_queries=Q, num_negatives=Nn, temp=temp, strong_threshold=0.8, alpha=0.99)
+    _, _, c0, _, _ = run_loss(lib, "nograd-f32", rep0, label, mask, prob, protos, kw, seed)
+    a, n = c0.sample_indices(seed, 0)
+
+    def step():
+        rep = rep0.clone().requires_grad_(True)
+        crit = css_b200.Contrast_Loss(seed=seed, **kw).cuda()
+        p = protos.clone()
+        loss = crit(rep, label, mask, prob, p, _indices=(a, n))
+        loss.backward()
+        return loss, rep, crit, p
+    (loss, rep, crit, p), names = launched(step)
+    assert_launched(NHWC_LOSS_KERNELS, names)
+    assert crit.last["rows_cache_mode"] == "verify"
+    assert int(crit.last["ws"].meta[css_b200._lib.META_ROWS_STALE].item()) == 0
+    assert rep.grad.stride() == rep0.stride()
+    check_against_f64("grad-f32", loss, rep.grad, crit, protos, p, rep0, label, mask, kw, a, n, "nhwc")
+
+
+# ---------------------------------------------------------------------------------------------------------------------------
+# NCHW tensor-core rep pass (css_sim_tc.cu rep_pass_tc_kernel<ROWS, NP>, proto_prep_tc_kernel)
+# ---------------------------------------------------------------------------------------------------------------------------
+@pytest.fixture
+def tc_lib():
+    from css_b200 import _lib
+    lib = _lib.load()
+    lib.css_set_rep_pass_path(1)
+    yield lib
+    lib.css_set_rep_pass_path(-1)
+
+
+@pytest.mark.parametrize("C,shape,offset,temp,kernels", TC_CASES)
+def test_tc_rep_pass(tc_lib, C, shape, offset, temp, kernels):
+    """Cosine map, or softmax + rows + norms, with the map `offset` floats into its buffer."""
+    import css_b200
+    B, h, w = TC_SHAPES[shape]
+    x, protos = rich_map(B, h, w, C, seed=7000 + 100 * C + 10 * offset + h)
+    buf = torch.full((x.numel() + 4,), float("nan"), device="cuda")
+    rep = buf[offset:offset + x.numel()].view(x.shape)
+    rep.copy_(x)
+    assert rep.data_ptr() % 16 == 4 * offset
+    if temp is None:
+        out, names = launched(lambda: css_b200.ops.cos_sim_map(rep, protos))
+    else:
+        out, names = launched(lambda: css_b200.ops.proto_softmax_sim(rep, protos, temp))
+    assert_launched(kernels, names)
+    check_sim_map(out, x, protos, temp, "tc")
+    if temp is not None:
+        assert torch.equal(out._css_rows.rows, x.permute(0, 2, 3, 1).reshape(-1, 256))
+        check_norms(out._css_rows.norms, x, "tc")
 
 
 # ---------------------------------------------------------------------------------------------------------------------------

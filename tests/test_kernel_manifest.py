@@ -40,15 +40,6 @@ COVERED_ELSEWHERE = {
     "ohem_scan_kernel<2>": "tests/test_gpu_ohem.py::test_cityscapes_full_size",
     "ohem_select_sum_kernel": "tests/test_gpu_ohem.py::test_cityscapes_full_size",
     "ohem_finalize_kernel": "tests/test_gpu_ohem.py::test_cityscapes_full_size",
-    "proto_prep_tc_kernel": "tests/test_gpu_stage12.py::test_tensor_core_rep_pass_matches_oracle_and_fma_path",
-    "rep_pass_tc_kernel<false, 3>": "tests/test_gpu_stage12.py::test_tensor_core_rep_pass_matches_oracle_and_fma_path",
-    "rep_pass_tc_kernel<true, 3>": "tests/test_gpu_stage12.py::test_tensor_core_rep_pass_matches_oracle_and_fma_path",
-    "rep_pass_tc_kernel<false, 4>": "tests/test_gpu_stage12.py::test_tensor_core_rep_pass_matches_oracle_and_fma_path",
-    "rep_pass_tc_kernel<true, 4>": "tests/test_gpu_stage12.py::test_tensor_core_rep_pass_matches_oracle_and_fma_path",
-    "rep_pass_nhwc_kernel<3>": "tests/test_gpu_nhwc.py::test_similarity_maps_from_channels_last",
-    "rep_pass_nhwc_kernel<4>": "tests/test_gpu_nhwc.py::test_similarity_maps_from_channels_last",
-    "rows_verify_rm_kernel": "tests/test_gpu_nhwc.py::test_channels_last_cache_modes_and_fallbacks",
-    "grad_rows_kernel": "tests/test_gpu_nhwc.py::test_contrast_loss_on_channels_last_map",
     "grad_scatter_kernel": "tests/test_gpu_grad.py::test_grad_scatter_matches_numpy",
     "rows_verify_kernel<float>": "tests/test_gpu_ddp.py::test_rows_cache_never_serves_stale_rows",
     "sample_kernel": "tests/test_gpu_loss.py::test_contrast_loss_against_oracle_device_draws",
