@@ -230,50 +230,22 @@ struct QueryShared {                     // per-CTA scratch for merging the SC_W
     float m[SC_WARPS], l[SC_WARPS], pos[2];
 };
 
-// Merge the four 8-lane groups of every warp, then the SC_WARPS warps (fixed order), and write the query's loss, anchor
-// pixel and d loss / d anchor.
+// Publish a warp's state (m, l: lane 0; its slice of sum 2^{z-m} r_hat: already in sh.acc[warp]; the positive's logit and
+// cosine: already in sh.pos), then merge the SC_WARPS warps in warp order and write the query's loss, anchor pixel and
+// d loss / d anchor.
 template <bool WANT_GRAD, typename RT>
-__device__ __forceinline__ void finish_query(Online& st, float z0, float cos_pos, QueryShared& sh, const RT* __restrict__ rows,
+__device__ __forceinline__ void finish_warps(float m, float l_w, QueryShared& sh, const RT* __restrict__ rows,
                                              const float4* __restrict__ proto_hat, float inv_na, int pa, int c, int k, int q, int Q,
                                              int V, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px,
                                              float4* __restrict__ grad_anchor) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int grp = lane >> 3, l8 = lane & 7;
     float4 (&s_acc)[SC_WARPS][CSS_D / 4] = sh.acc;
     float (&s_m)[SC_WARPS] = sh.m;
     float (&s_l)[SC_WARPS] = sh.l;
     float (&s_pos)[2] = sh.pos;
-    // merge the four groups (xor 8, xor 16); afterwards every lane holds the warp's state for its column slice
-#pragma unroll
-    for (int o = 8; o <= 16; o <<= 1) {
-        const float m_o = __shfl_xor_sync(0xffffffffu, st.m, o);
-        const float l_o = __shfl_xor_sync(0xffffffffu, st.l, o);
-        const float M = fmaxf(st.m, m_o);
-        const float s_a = (st.m == -INFINITY) ? 0.f : exp2f(st.m - M);
-        const float s_b = (m_o == -INFINITY) ? 0.f : exp2f(m_o - M);
-        st.l = st.l * s_a + l_o * s_b;
-        if (WANT_GRAD) {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                st.acc[i].x = st.acc[i].x * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].x, o) * s_b;
-                st.acc[i].y = st.acc[i].y * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].y, o) * s_b;
-                st.acc[i].z = st.acc[i].z * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].z, o) * s_b;
-                st.acc[i].w = st.acc[i].w * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].w, o) * s_b;
-            }
-        }
-        st.m = M;
-    }
     if (lane == 0) {
-        s_m[warp] = st.m;
-        s_l[warp] = st.l;
-        if (warp == 0) {
-            s_pos[0] = z0;
-            s_pos[1] = cos_pos;
-        }
-    }
-    if (WANT_GRAD && grp == 0) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) s_acc[warp][i * 8 + l8] = st.acc[i];
+        s_m[warp] = m;
+        s_l[warp] = l_w;
     }
     __syncthreads();
     if (warp != 0) return;
@@ -334,6 +306,47 @@ __device__ __forceinline__ void finish_query(Online& st, float z0, float cos_pos
     }
 }
 
+// Merge the four 8-lane groups of every warp, then the SC_WARPS warps (fixed order), and write the query's loss, anchor
+// pixel and d loss / d anchor.
+template <bool WANT_GRAD, typename RT>
+__device__ __forceinline__ void finish_query(Online& st, float z0, float cos_pos, QueryShared& sh, const RT* __restrict__ rows,
+                                             const float4* __restrict__ proto_hat, float inv_na, int pa, int c, int k, int q, int Q,
+                                             int V, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px,
+                                             float4* __restrict__ grad_anchor) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int grp = lane >> 3, l8 = lane & 7;
+    // merge the four groups (xor 8, xor 16); afterwards every lane holds the warp's state for its column slice
+#pragma unroll
+    for (int o = 8; o <= 16; o <<= 1) {
+        const float m_o = __shfl_xor_sync(0xffffffffu, st.m, o);
+        const float l_o = __shfl_xor_sync(0xffffffffu, st.l, o);
+        const float M = fmaxf(st.m, m_o);
+        const float s_a = (st.m == -INFINITY) ? 0.f : exp2f(st.m - M);
+        const float s_b = (m_o == -INFINITY) ? 0.f : exp2f(m_o - M);
+        st.l = st.l * s_a + l_o * s_b;
+        if (WANT_GRAD) {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                st.acc[i].x = st.acc[i].x * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].x, o) * s_b;
+                st.acc[i].y = st.acc[i].y * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].y, o) * s_b;
+                st.acc[i].z = st.acc[i].z * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].z, o) * s_b;
+                st.acc[i].w = st.acc[i].w * s_a + __shfl_xor_sync(0xffffffffu, st.acc[i].w, o) * s_b;
+            }
+        }
+        st.m = M;
+    }
+    if (WANT_GRAD && grp == 0) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) sh.acc[warp][i * 8 + l8] = st.acc[i];
+    }
+    if (threadIdx.x == 0) {
+        sh.pos[0] = z0;
+        sh.pos[1] = cos_pos;
+    }
+    finish_warps<WANT_GRAD, RT>(st.m, st.l, sh, rows, proto_hat, inv_na, pa, c, k, q, Q, V, temp, loss_kq, anchor_px,
+                                grad_anchor);
+}
+
 // publishes the Philox offset of this call, offset + *step_counter, into meta and bumps the device-resident counter so the
 // next call -- or the next replay of a captured CUDA graph -- draws fresh samples
 __global__ void draw_offset_kernel(uint64_t offset, unsigned long long* __restrict__ step_counter, int32_t* __restrict__ meta) {
@@ -369,8 +382,167 @@ __device__ __forceinline__ void load_candidate(const RT* __restrict__ rows, cons
     }
 }
 
+// ids of the warp's candidates 32 b + lane: negative j - 1 = warp + SC_WARPS n  ->  pixel-major row, or -2 past the end
+template <bool FED>
+__device__ __forceinline__ int ring_candidate_row(const SlotTables& tb, const DrawKey& dk, const int32_t* __restrict__ neg_idx,
+                                                  const int32_t* __restrict__ valid_list, int k, int q, int Q, int Nn, int N, int n, int cnt) {
+    if (n >= cnt) return -2;
+    const int jm1 = (threadIdx.x >> 5) + SC_WARPS * n;
+    int seg, within;
+    if (FED) {
+        const int idx = neg_idx[((size_t)k * Q + q) * Nn + jm1];
+        seg = upper_bound32(tb.rot_off + 1, idx);
+        within = idx - tb.rot_off[seg];
+    } else {
+        within = draw_negative(dk, k, q, jm1, tb.cdf, tb.rot_off, seg);
+    }
+    return valid_list[(size_t)tb.rot_cls[seg] * N + within];
+}
+
+// -------------------------------------------------------------------------------------------------------------------
+// Whole-warp rows: every candidate row is spread over the 32 lanes (lane l holds float4 l and l + 32 of the 1 KB row), so the
+// anchor slice and the gradient accumulator take 8 registers each, once per warp, instead of one full copy per 8-lane group.
+// The registers this frees hold R rows per warp in flight: per batch, 2R back-to-back LDG.128 per lane.  The R partial dots
+// are reduced by a transpose-reduce (xor 16 halves the values a lane holds, then xor 8, ..., until one is left; the last
+// offsets finish the sum), which leaves the full dot of row lane / (32 / R) on every lane: about one shuffle per row
+// instead of five, and one exp2 per lane covers the batch.  Each row's weight 2^{z-m} / ||r|| is then broadcast with one
+// shuffle and the rows are accumulated with 4 FFMA2 per row.  The online-max variant (!FIX) takes one warp max per batch.
+// -------------------------------------------------------------------------------------------------------------------
+template <int R>
+__device__ __forceinline__ float transpose_sum(float (&d)[R], int lane) {
+#pragma unroll
+    for (int o = 16, n = R; n > 1; o >>= 1, n >>= 1) {
+        const bool up = lane & o;
+#pragma unroll
+        for (int i = 0; i < n / 2; ++i) {
+            const float send = up ? d[i] : d[i + n / 2];
+            const float keep = up ? d[i + n / 2] : d[i];
+            d[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+        }
+    }
+    float v = d[0];
+#pragma unroll
+    for (int o = 16 / R; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+__device__ __forceinline__ float2 dot2x4(const float4& a0, const float4& a1, const float4& r0, const float4& r1) {
+    float2 s = __fmul2_rn(lo2(a0), lo2(r0));
+    s = __ffma2_rn(hi2(a0), hi2(r0), s);
+    s = __ffma2_rn(lo2(a1), lo2(r1), s);
+    return __ffma2_rn(hi2(a1), hi2(r1), s);
+}
+
+__device__ __forceinline__ void axpy4(float wr, const float4& r, float4& acc) {
+    const float2 ww = make_float2(wr, wr);
+    const float2 lo = __ffma2_rn(ww, lo2(r), lo2(acc));
+    const float2 hi = __ffma2_rn(ww, hi2(r), hi2(acc));
+    acc = make_float4(lo.x, lo.y, hi.x, hi.y);
+}
+
+// The fp32 gradient form of score_ce_kernel, after the slot tables and the anchor pixel `pa` are known (R rows per batch).
+template <bool FIX, int R>
+__device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, const float* __restrict__ norms, const float4* __restrict__ proto_hat,
+                                                const int32_t* __restrict__ valid_list, const int32_t* __restrict__ neg_idx,
+                                                const SlotTables& tb, QueryShared& sh, const DrawKey& dk, int pa, int c, int k, int q, int N,
+                                                int Q, int Nn, int V, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px,
+                                                float4* __restrict__ grad_anchor) {
+    static_assert(R == 2 || R == 4 || R == 8 || R == 16, "R rows per batch, a power of two that divides the 32-id batch");
+    constexpr int LPR = 32 / R;                                // lanes that end up holding one row's dot
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    // warp w owns the negatives j - 1 = w + SC_WARPS n, n < cnt; their ids come 32 at a time, one per lane
+    const int cnt = (Nn - warp + SC_WARPS - 1) / SC_WARPS;
+    int cur_row = (neg_idx ? ring_candidate_row<true>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt)
+                             : ring_candidate_row<false>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt));
+
+    const float4* rows4 = reinterpret_cast<const float4*>(rows);
+    const float4 a0 = __ldg(rows4 + (size_t)pa * (CSS_D / 4) + lane), a1 = __ldg(rows4 + (size_t)pa * (CSS_D / 4) + 32 + lane);
+    const float inv_na = 1.f / fmaxf(norms[pa], 1e-8f);       // cosine_similarity eps (loss.py:146)
+    const float scale2 = 1.4426950408889634f / temp;
+    float cur_inv = 1.f / fmaxf(norms[max(cur_row, 0)], 1e-8f);
+
+    // candidate 0 = the (updated) prototype of class c (loss.py:143-144): scored by every warp, kept by warp 0
+    float4 acc0, acc1;
+    float m, l;                                                // l: this lane's share (one lane per row adds its weight)
+    {
+        const float4* pp = proto_hat + (size_t)c * (CSS_D / 4);
+        const float4 p0 = __ldg(pp + lane), p1 = __ldg(pp + 32 + lane);
+        const float2 s = dot2x4(a0, a1, p0, p1);
+        const float cos_pos = warp_sum(s.x + s.y) * inv_na;
+        const float z0 = cos_pos * scale2;
+        m = FIX ? scale2 : (warp == 0 ? z0 : -INFINITY);
+        const float w0 = (warp == 0) ? exp2f(z0 - m) : 0.f;
+        l = (lane == 0) ? w0 : 0.f;
+        acc0 = make_float4(w0 * p0.x, w0 * p0.y, w0 * p0.z, w0 * p0.w);
+        acc1 = make_float4(w0 * p1.x, w0 * p1.y, w0 * p1.z, w0 * p1.w);
+        if (threadIdx.x == 0) {                                // read by finish_warps after its barrier
+            sh.pos[0] = z0;
+            sh.pos[1] = cos_pos;
+        }
+    }
+
+#pragma unroll 1
+    for (int base = 0; base < cnt; base += 32) {
+        const int nxt_row = neg_idx ? ring_candidate_row<true>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, base + 32 + lane, cnt)
+                                    : ring_candidate_row<false>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, base + 32 + lane, cnt);
+        const int n_batches = min(32, cnt - base + R - 1) / R;
+        float nxt_nrm = 1.f;
+#pragma unroll 1
+        for (int t = 0; t < n_batches; ++t) {
+            float4 r[R][2];
+#pragma unroll
+            for (int i = 0; i < R; ++i) {                      // past the end: row 0 (any finite row), weight 0
+                const float4* p = rows4 + (size_t)max(__shfl_sync(0xffffffffu, cur_row, t * R + i), 0) * (CSS_D / 4) + lane;
+                r[i][0] = __ldg(p);
+                r[i][1] = __ldg(p + 32);
+            }
+            float d[R];
+#pragma unroll
+            for (int i = 0; i < R; ++i) {
+                const float2 s = dot2x4(a0, a1, r[i][0], r[i][1]);
+                d[i] = s.x + s.y;
+            }
+            const int mine = t * R + lane / LPR;               // the candidate whose dot this lane ends up with
+            const float inv = __shfl_sync(0xffffffffu, cur_inv, mine);
+            const float z = transpose_sum<R>(d, lane) * (inv_na * inv) * scale2;
+            const bool valid = base + mine < cnt;
+            if (!FIX) {
+                float zm = valid ? z : -INFINITY;
+#pragma unroll
+                for (int o = LPR; o < 32; o <<= 1) zm = fmaxf(zm, __shfl_xor_sync(0xffffffffu, zm, o));
+                if (zm > m) {                                  // warp-uniform
+                    const float sc = exp2f(m - zm);            // m = -inf -> 0
+                    l *= sc;
+                    acc0 = make_float4(acc0.x * sc, acc0.y * sc, acc0.z * sc, acc0.w * sc);
+                    acc1 = make_float4(acc1.x * sc, acc1.y * sc, acc1.z * sc, acc1.w * sc);
+                    m = zm;
+                }
+            }
+            const float wgt = valid ? exp2f(z - m) : 0.f;
+            if (lane % LPR == 0) l += wgt;
+            const float wr = wgt * inv;
+#pragma unroll
+            for (int i = 0; i < R; ++i) {
+                const float wi = __shfl_sync(0xffffffffu, wr, i * LPR);
+                axpy4(wi, r[i][0], acc0);
+                axpy4(wi, r[i][1], acc1);
+            }
+            if (t == 0) nxt_nrm = norms[max(nxt_row, 0)];      // the id has landed by now; used after the batch
+        }
+        cur_row = nxt_row;
+        cur_inv = 1.f / fmaxf(nxt_nrm, 1e-8f);
+    }
+    sh.acc[warp][lane] = acc0;
+    sh.acc[warp][lane + 32] = acc1;
+    finish_warps<true, float>(m, warp_sum(l), sh, rows, proto_hat, inv_na, pa, c, k, q, Q, V, temp, loss_kq, anchor_px,
+                              grad_anchor);
+}
+
+
+// fp32 rows with the gradient take the whole-warp layout above (8 rows per batch, 4 CTAs/SM; PREFETCH and ASMEM select among
+// the forms of the 8-lane-group layout, which the bf16 and forward-only variants keep)
 template <bool WANT_GRAD, bool PREFETCH, bool ASMEM, bool FIX, typename RT>
-__global__ void __launch_bounds__(SC_THREADS, (WANT_GRAD && !ASMEM) ? 4 : 5) score_ce_kernel(
+__global__ void __launch_bounds__(SC_THREADS, (WANT_GRAD && (!ASMEM || sizeof(RT) == 4)) ? 4 : 5) score_ce_kernel(
     const RT* __restrict__ rows, const float* __restrict__ norms, const float4* __restrict__ proto_hat,
     const float* __restrict__ class_cdf, const int32_t* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
     const int32_t* __restrict__ meta, const int32_t* __restrict__ anchor_idx, const int32_t* __restrict__ neg_idx, uint64_t seed,
@@ -396,6 +568,11 @@ __global__ void __launch_bounds__(SC_THREADS, (WANT_GRAD && !ASMEM) ? 4 : 5) sco
     const DrawKey dk = make_key(seed, ((uint64_t)(uint32_t)meta[CSS_META_DRAW_OFFSET + 1] << 32) | (uint32_t)meta[CSS_META_DRAW_OFFSET]);
     const int ai = anchor_idx ? anchor_idx[k * Q + q] : draw_anchor(dk, k, q, n_hard);
     const int pa = hard_list[(size_t)c * N + ai];
+    if constexpr (WANT_GRAD && sizeof(RT) == 4) {
+        score_rows_wide<FIX, 8>(rows, norms, proto_hat, valid_list, neg_idx, tb, sh, dk, pa, c, k, q, N, Q, Nn, V, temp, loss_kq, anchor_px,
+                                grad_anchor);
+        return;
+    }
     __shared__ float4 s_a[ASMEM ? CSS_D / 4 : 1];
     float4 a[ASMEM ? 1 : 8];
     if (ASMEM) {
@@ -505,23 +682,6 @@ template <int N_PENDING>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N_PENDING) : "memory"); }
 
 #define RING_STAGE_BYTES (4 * CSS_D * 4)          // four fp32 rows, one per 8-lane group
-
-// ids of the warp's candidates 32 b + lane: negative j - 1 = warp + SC_WARPS n  ->  pixel-major row, or -2 past the end
-template <bool FED>
-__device__ __forceinline__ int ring_candidate_row(const SlotTables& tb, const DrawKey& dk, const int32_t* __restrict__ neg_idx,
-                                                  const int32_t* __restrict__ valid_list, int k, int q, int Q, int Nn, int N, int n, int cnt) {
-    if (n >= cnt) return -2;
-    const int jm1 = (threadIdx.x >> 5) + SC_WARPS * n;
-    int seg, within;
-    if (FED) {
-        const int idx = neg_idx[((size_t)k * Q + q) * Nn + jm1];
-        seg = upper_bound32(tb.rot_off + 1, idx);
-        within = idx - tb.rot_off[seg];
-    } else {
-        within = draw_negative(dk, k, q, jm1, tb.cdf, tb.rot_off, seg);
-    }
-    return valid_list[(size_t)tb.rot_cls[seg] * N + within];
-}
 
 template <bool FIX, bool FED, int STAGES, int MINB>
 __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_ring_kernel(
@@ -807,10 +967,12 @@ __global__ void __launch_bounds__(256) loss_reduce_kernel(const float* __restric
     }
 }
 
-// which kernel scores fp32 rows with the gradient: 0 = register kernel, 1 = shared-memory ring (2 stages, cp.async),
-// 2 = register / bulk-copy hybrid (default: faster than the register kernel at 28 of the 30 configs[4] points, -2 % of the step on average); css_set_scorer_path() overrides CSS_B200_SCORER=reg|ring|bulk, which overrides the default
+// which kernel scores fp32 rows with the gradient: 0 = register kernel (default: whole-warp rows, 8 rows per batch in flight per
+// warp at 4 CTAs/SM, the most the 128-register budget holds without spills; the 5376 CTAs of the bench shape make 9.08 waves),
+// 1 = shared-memory ring (2 stages, cp.async), 2 = register / bulk-copy hybrid on 8-lane groups; css_set_scorer_path() overrides
+// CSS_B200_SCORER=reg|ring|bulk, which overrides the default
 #ifndef CSS_SCORER_DEFAULT
-#define CSS_SCORER_DEFAULT 2
+#define CSS_SCORER_DEFAULT 0
 #endif
 static int g_scorer_path = -1;
 extern "C" int css_set_scorer_path(int path) {
