@@ -33,7 +33,8 @@ SIGNATURES = {
     "css_sim_map": (c_int, [P, c_int, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_float, P, P]),
     "css_upsample_label_fuse": (c_int, [P, P, c_float, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, P, P, P, P, P]),
     "css_select_tiles": (c_int, [c_int]),
-    "css_select": (c_int, [P, P, P, c_float, c_int, c_int, c_int, c_int, P, P, P, P, P, P, P]),
+    "css_select": (c_int, [P, P, P, c_float, c_int, c_int, c_int, c_int, P, P, P, P, P]),
+    "css_select_lists": (c_int, [P, P, P, P, c_int, c_int, P, P, P]),
     "css_rep_pass": (c_int, [P, c_int, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_float, P, P, P, P]),
     "css_set_rep_pass_path": (c_int, [c_int]),
     "css_set_scorer_path": (c_int, [c_int]),

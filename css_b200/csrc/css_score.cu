@@ -3,7 +3,8 @@
 // Reference: generalframeworks/loss/loss.py:124-149 (+ negative_index_sampler :410-418) and its autograd backward.
 //
 // Every query draws its own Nn negatives (loss.py:137-142), so this is a per-query row gather (1 KB fp32 rows of the
-// pixel-major copy written by css_rep_pass, scaled by 1/max(||r||,1e-8) on the fly), not a shared-operand GEMM: 2*D flops per 4*D gathered bytes.
+// pixel-major copy written by css_rep_pass, scaled on the fly by the 1/max(||r||,1e-8) that each valid-list entry carries next to its
+// pixel id), not a shared-operand GEMM: 2*D flops per 4*D gathered bytes.
 // It is bound by the L2 -> SM gather path (the 107 MB copy is mostly L2 resident at VOC size), not by the tensor pipe.
 //
 // Work split: one CTA (4 warps) per (present-class slot k, query q); warp w owns candidates j = w, w+4, ...  A warp is
@@ -11,7 +12,7 @@
 // line read by exactly one group), reduces the dot with 3 shuffles and keeps an online-softmax state
 // (m, l, sum_j 2^{z_j-m} r_hat_j) in registers, so the backward never re-gathers.  Packed fp32x2 FMAs (FFMA2, sm_100)
 // halve the FMA issue slots of the dot and of the weighted row accumulation.  Candidate row ids for the next 32
-// candidates are produced one per lane (Philox draw or fed index -> rotated segment -> class list lookup) and handed to
+// candidates are produced one per lane (Philox draw or fed index -> rotated segment -> one 8-byte class-list entry) and handed to
 // the groups by shuffle.  The four warp states are merged through shared memory in a fixed order (deterministic).
 #include "css_common.cuh"
 #include <stdlib.h>
@@ -382,11 +383,12 @@ __device__ __forceinline__ void load_candidate(const RT* __restrict__ rows, cons
     }
 }
 
-// ids of the warp's candidates 32 b + lane: negative j - 1 = warp + SC_WARPS n  ->  pixel-major row, or -2 past the end
+// ids of the warp's candidates 32 b + lane: negative j - 1 = warp + SC_WARPS n  ->  its valid-list entry {pixel-major row, bits of
+// 1 / max(||row||, 1e-8)}, or {-2, bits of 1} past the end (any finite inverse: those candidates carry weight 0)
 template <bool FED>
-__device__ __forceinline__ int ring_candidate_row(const SlotTables& tb, const DrawKey& dk, const int32_t* __restrict__ neg_idx,
-                                                  const int32_t* __restrict__ valid_list, int k, int q, int Q, int Nn, int N, int n, int cnt) {
-    if (n >= cnt) return -2;
+__device__ __forceinline__ int2 ring_candidate_row(const SlotTables& tb, const DrawKey& dk, const int32_t* __restrict__ neg_idx,
+                                                   const int2* __restrict__ valid_list, int k, int q, int Q, int Nn, int N, int n, int cnt) {
+    if (n >= cnt) return make_int2(-2, __float_as_int(1.f));
     const int jm1 = (threadIdx.x >> 5) + SC_WARPS * n;
     int seg, within;
     if (FED) {
@@ -405,8 +407,9 @@ __device__ __forceinline__ int ring_candidate_row(const SlotTables& tb, const Dr
 // The registers this frees hold R rows per warp in flight: per batch, 2R back-to-back LDG.128 per lane.  The R partial dots
 // are reduced by a transpose-reduce (xor 16 halves the values a lane holds, then xor 8, ..., until one is left; the last
 // offsets finish the sum), which leaves the full dot of row lane / (32 / R) on every lane: about one shuffle per row
-// instead of five, and one exp2 per lane covers the batch.  Each row's weight 2^{z-m} / ||r|| is then broadcast with one
-// shuffle and the rows are accumulated with 4 FFMA2 per row.  The online-max variant (!FIX) takes one warp max per batch.
+// instead of five, and one exp2 per lane covers the batch.  The batch's row ids and weights 2^{z-m} / ||r|| reach every lane
+// through a few words of shared memory (one broadcast LDS.128 per four values: shuffles, one per value, cost the same MIO
+// slots as these loads), and the rows are accumulated with 4 FFMA2 per row.  The online-max variant (!FIX) takes one warp max per batch.
 // -------------------------------------------------------------------------------------------------------------------
 template <int R>
 __device__ __forceinline__ float transpose_sum(float (&d)[R], int lane) {
@@ -443,7 +446,7 @@ __device__ __forceinline__ void axpy4(float wr, const float4& r, float4& acc) {
 // The fp32 gradient form of score_ce_kernel, after the slot tables and the anchor pixel `pa` are known (R rows per batch).
 template <bool FIX, int R>
 __device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, const float* __restrict__ norms, const float4* __restrict__ proto_hat,
-                                                const int32_t* __restrict__ valid_list, const int32_t* __restrict__ neg_idx,
+                                                const int2* __restrict__ valid_list, const int32_t* __restrict__ neg_idx,
                                                 const SlotTables& tb, QueryShared& sh, const DrawKey& dk, int pa, int c, int k, int q, int N,
                                                 int Q, int Nn, int V, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px,
                                                 float4* __restrict__ grad_anchor) {
@@ -452,14 +455,13 @@ __device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     // warp w owns the negatives j - 1 = w + SC_WARPS n, n < cnt; their ids come 32 at a time, one per lane
     const int cnt = (Nn - warp + SC_WARPS - 1) / SC_WARPS;
-    int cur_row = (neg_idx ? ring_candidate_row<true>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt)
-                             : ring_candidate_row<false>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt));
+    int2 cur = (neg_idx ? ring_candidate_row<true>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt)
+                        : ring_candidate_row<false>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt));
 
     const float4* rows4 = reinterpret_cast<const float4*>(rows);
     const float4 a0 = __ldg(rows4 + (size_t)pa * (CSS_D / 4) + lane), a1 = __ldg(rows4 + (size_t)pa * (CSS_D / 4) + 32 + lane);
     const float inv_na = 1.f / fmaxf(norms[pa], 1e-8f);       // cosine_similarity eps (loss.py:146)
     const float scale2 = 1.4426950408889634f / temp;
-    float cur_inv = 1.f / fmaxf(norms[max(cur_row, 0)], 1e-8f);
 
     // candidate 0 = the (updated) prototype of class c (loss.py:143-144): scored by every warp, kept by warp 0
     float4 acc0, acc1;
@@ -481,18 +483,30 @@ __device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, 
         }
     }
 
+    // the id group's row ids and each batch's weights reach every lane through the warp's words of shared memory: one
+    // broadcast LDS.128 per four values instead of one shuffle per value
+    __shared__ __align__(16) int s_id[SC_WARPS][32];
+    __shared__ __align__(16) float s_w[SC_WARPS][R];
 #pragma unroll 1
     for (int base = 0; base < cnt; base += 32) {
-        const int nxt_row = neg_idx ? ring_candidate_row<true>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, base + 32 + lane, cnt)
-                                    : ring_candidate_row<false>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, base + 32 + lane, cnt);
+        const int2 nxt = neg_idx ? ring_candidate_row<true>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, base + 32 + lane, cnt)
+                                 : ring_candidate_row<false>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, base + 32 + lane, cnt);
         const int n_batches = min(32, cnt - base + R - 1) / R;
-        float nxt_nrm = 1.f;
+        __syncwarp();                                          // the previous group's ids have been read
+        s_id[warp][lane] = cur.x;
+        __syncwarp();
 #pragma unroll 1
         for (int t = 0; t < n_batches; ++t) {
             float4 r[R][2];
+            int ids[R];
+#pragma unroll
+            for (int i = 0; i < R; i += 4) {
+                const int4 v = *reinterpret_cast<const int4*>(&s_id[warp][t * R + i]);
+                ids[i] = v.x; ids[i + 1] = v.y; ids[i + 2] = v.z; ids[i + 3] = v.w;
+            }
 #pragma unroll
             for (int i = 0; i < R; ++i) {                      // past the end: row 0 (any finite row), weight 0
-                const float4* p = rows4 + (size_t)max(__shfl_sync(0xffffffffu, cur_row, t * R + i), 0) * (CSS_D / 4) + lane;
+                const float4* p = rows4 + (size_t)max(ids[i], 0) * (CSS_D / 4) + lane;
                 r[i][0] = __ldg(p);
                 r[i][1] = __ldg(p + 32);
             }
@@ -503,7 +517,7 @@ __device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, 
                 d[i] = s.x + s.y;
             }
             const int mine = t * R + lane / LPR;               // the candidate whose dot this lane ends up with
-            const float inv = __shfl_sync(0xffffffffu, cur_inv, mine);
+            const float inv = __int_as_float(__shfl_sync(0xffffffffu, cur.y, mine));
             const float z = transpose_sum<R>(d, lane) * (inv_na * inv) * scale2;
             const bool valid = base + mine < cnt;
             if (!FIX) {
@@ -521,16 +535,22 @@ __device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, 
             const float wgt = valid ? exp2f(z - m) : 0.f;
             if (lane % LPR == 0) l += wgt;
             const float wr = wgt * inv;
+            float w[R];
+            if (lane % LPR == 0) s_w[warp][lane / LPR] = wr;
+            __syncwarp();
+#pragma unroll
+            for (int i = 0; i < R; i += 4) {
+                const float4 v = *reinterpret_cast<const float4*>(&s_w[warp][i]);
+                w[i] = v.x; w[i + 1] = v.y; w[i + 2] = v.z; w[i + 3] = v.w;
+            }
+            __syncwarp();                                      // read before the next batch writes
 #pragma unroll
             for (int i = 0; i < R; ++i) {
-                const float wi = __shfl_sync(0xffffffffu, wr, i * LPR);
-                axpy4(wi, r[i][0], acc0);
-                axpy4(wi, r[i][1], acc1);
+                axpy4(w[i], r[i][0], acc0);
+                axpy4(w[i], r[i][1], acc1);
             }
-            if (t == 0) nxt_nrm = norms[max(nxt_row, 0)];      // the id has landed by now; used after the batch
         }
-        cur_row = nxt_row;
-        cur_inv = 1.f / fmaxf(nxt_nrm, 1e-8f);
+        cur = nxt;
     }
     sh.acc[warp][lane] = acc0;
     sh.acc[warp][lane + 32] = acc1;
@@ -544,7 +564,7 @@ __device__ __forceinline__ void score_rows_wide(const float* __restrict__ rows, 
 template <bool WANT_GRAD, bool PREFETCH, bool ASMEM, bool FIX, typename RT>
 __global__ void __launch_bounds__(SC_THREADS, (WANT_GRAD && (!ASMEM || sizeof(RT) == 4)) ? 4 : 5) score_ce_kernel(
     const RT* __restrict__ rows, const float* __restrict__ norms, const float4* __restrict__ proto_hat,
-    const float* __restrict__ class_cdf, const int32_t* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
+    const float* __restrict__ class_cdf, const int2* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
     const int32_t* __restrict__ meta, const int32_t* __restrict__ anchor_idx, const int32_t* __restrict__ neg_idx, uint64_t seed,
     int N, int Q, int Nn, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px, float4* __restrict__ grad_anchor) {
     css_pdl_enter();
@@ -615,8 +635,9 @@ __global__ void __launch_bounds__(SC_THREADS, (WANT_GRAD && (!ASMEM || sizeof(RT
                 } else {
                     within = draw_negative(dk, k, q, j - 1, tb.cdf, tb.rot_off, seg);
                 }
-                my_row = valid_list[(size_t)tb.rot_cls[seg] * N + within];
-                my_inv = 1.f / fmaxf(norms[my_row], 1e-8f);
+                const int2 e = valid_list[(size_t)tb.rot_cls[seg] * N + within];
+                my_row = e.x;
+                my_inv = __int_as_float(e.y);
             }
         }
         const int steps = min(8, (cnt - base + 3) >> 2);
@@ -686,7 +707,7 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 template <bool FIX, bool FED, int STAGES, int MINB>
 __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_ring_kernel(
     const float* __restrict__ rows, const float* __restrict__ norms, const float4* __restrict__ proto_hat,
-    const float* __restrict__ class_cdf, const int32_t* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
+    const float* __restrict__ class_cdf, const int2* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
     const int32_t* __restrict__ meta, const int32_t* __restrict__ anchor_idx, const int32_t* __restrict__ neg_idx, uint64_t seed,
     int N, int Q, int Nn, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px, float4* __restrict__ grad_anchor) {
     css_pdl_enter();
@@ -714,8 +735,8 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_ring_kernel(
     // warp w owns the negatives j - 1 = w + SC_WARPS n, n < cnt, four per step (one per group)
     const int cnt = (Nn - warp + SC_WARPS - 1) / SC_WARPS;
     const int T = (cnt + 3) >> 2;
-    int cur_row = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt);
-    int nxt_row = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, 32 + lane, cnt);
+    int2 cur = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt);
+    int2 nxt = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, 32 + lane, cnt);
 
     // this lane's 16-byte chunks of the ring: stage s, chunk i at lane_base + s * RING_STAGE_BYTES + i * 128
     const uint32_t ring0 = (uint32_t)__cvta_generic_to_shared(ring_smem) + warp * (STAGES * RING_STAGE_BYTES) + grp * (CSS_D * 4) + l8 * 16;
@@ -728,7 +749,7 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_ring_kernel(
     uint32_t wr_off = 0, rd_off = 0;
 #pragma unroll
     for (int p = 0; p < STAGES - 1; ++p) {
-        issue(wr_off, __shfl_sync(0xffffffffu, cur_row, p * 4 + grp));
+        issue(wr_off, __shfl_sync(0xffffffffu, cur.x, p * 4 + grp));
         cp_async_commit();
         wr_off += RING_STAGE_BYTES;
     }
@@ -738,7 +759,6 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_ring_kernel(
     for (int i = 0; i < 8; ++i) a[i] = row_f4(rows, (size_t)pa, i * 8 + l8);
     const float inv_na = 1.f / fmaxf(norms[pa], 1e-8f);       // cosine_similarity eps (loss.py:146)
     const float scale2 = 1.4426950408889634f / temp;
-    float cur_inv = 1.f / fmaxf(norms[max(cur_row, 0)], 1e-8f);
 
     Online st;
     st.m = FIX ? scale2 : -INFINITY;
@@ -762,30 +782,27 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_ring_kernel(
     // end carry weight 0 and copy row 0 (the loop has a single exit, which keeps the accumulators out of local memory).
 #pragma unroll 1
     for (int b = 0; b * 8 < T; ++b) {
-        float nxt_nrm = 1.f;
 #pragma unroll 1
         for (int t = 0; t < 8; ++t) {
             {   // copies of step s + STAGES - 1
                 const int tp = t + (STAGES - 1);
-                const int prow = __shfl_sync(0xffffffffu, (tp < 8) ? cur_row : nxt_row, (tp & 7) * 4 + grp);
+                const int prow = __shfl_sync(0xffffffffu, (tp < 8) ? cur.x : nxt.x, (tp & 7) * 4 + grp);
                 issue(wr_off, prow);
                 cp_async_commit();
                 wr_off = (wr_off + RING_STAGE_BYTES == STAGES * RING_STAGE_BYTES) ? 0u : wr_off + RING_STAGE_BYTES;
             }
             cp_async_wait<STAGES - 1>();
-            const int row = __shfl_sync(0xffffffffu, cur_row, t * 4 + grp);
-            const float inv = __shfl_sync(0xffffffffu, cur_inv, t * 4 + grp);
+            const int row = __shfl_sync(0xffffffffu, cur.x, t * 4 + grp);
+            const float inv = __int_as_float(__shfl_sync(0xffffffffu, cur.y, t * 4 + grp));
             float4 r[8];
 #pragma unroll
             for (int i = 0; i < 8; ++i) r[i] = lds128(ring0 + rd_off + i * 128);
             rd_off = (rd_off + RING_STAGE_BYTES == STAGES * RING_STAGE_BYTES) ? 0u : rd_off + RING_STAGE_BYTES;
             const float cosv = group_sum8(dot8(a, r)) * (inv_na * inv);
             online_update<true, FIX>(st, cosv * scale2, row >= 0, inv, r);
-            if (t == 3) nxt_nrm = norms[max(nxt_row, 0)];       // the id has landed by now; used after the batch
         }
-        cur_row = nxt_row;
-        cur_inv = 1.f / fmaxf(nxt_nrm, 1e-8f);
-        nxt_row = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, (b + 2) * 32 + lane, cnt);
+        cur = nxt;
+        nxt = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, (b + 2) * 32 + lane, cnt);
     }
     cp_async_wait<0>();
     finish_query<true, float>(st, z0, cos_pos, sh, rows, proto_hat, inv_na, pa, c, k, q, Q, V, temp, loss_kq, anchor_px, grad_anchor);
@@ -823,7 +840,7 @@ __device__ __forceinline__ void sc_bulk_g2s(uint32_t dst, const void* src, uint3
 template <bool FIX, bool FED, int PERIOD, int NBUF, int MINB>
 __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
     const float* __restrict__ rows, const float* __restrict__ norms, const float4* __restrict__ proto_hat,
-    const float* __restrict__ class_cdf, const int32_t* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
+    const float* __restrict__ class_cdf, const int2* __restrict__ valid_list, const int32_t* __restrict__ hard_list,
     const int32_t* __restrict__ meta, const int32_t* __restrict__ anchor_idx, const int32_t* __restrict__ neg_idx, uint64_t seed,
     int N, int Q, int Nn, float temp, float* __restrict__ loss_kq, int32_t* __restrict__ anchor_px, float4* __restrict__ grad_anchor) {
     static_assert(NBUF * PERIOD <= 8 && 8 % PERIOD == 0 && (8 / PERIOD) % NBUF == 0, "refill distance must stay inside the next id batch");
@@ -858,8 +875,8 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
 
     const int cnt = (Nn - warp + SC_WARPS - 1) / SC_WARPS;
     const int T = (cnt + 3) >> 2;
-    int cur_row = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt);
-    int nxt_row = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, 32 + lane, cnt);
+    int2 cur = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, lane, cnt);
+    int2 nxt = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, 32 + lane, cnt);
 
     const uint32_t grp_buf = (uint32_t)__cvta_generic_to_shared(stage_smem) + warp * (NBUF * RING_STAGE_BYTES) + grp * (CSS_D * 4);
     const uint32_t buf = grp_buf + l8 * 16;
@@ -868,14 +885,13 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
         if (l8 == 0) sc_bulk_g2s(grp_buf + ib * RING_STAGE_BYTES, reinterpret_cast<const char*>(rows) + (size_t)max(row, 0) * (CSS_D * 4), CSS_D * 4, bar0 + ib * 8);
     };
 #pragma unroll
-    for (int i = 0; i < NBUF; ++i) refill(i, __shfl_sync(0xffffffffu, cur_row, i * PERIOD * 4 + grp));
+    for (int i = 0; i < NBUF; ++i) refill(i, __shfl_sync(0xffffffffu, cur.x, i * PERIOD * 4 + grp));
 
     float4 a[8];                                               // the anchor stays in registers (128 registers, 4 CTAs/SM)
 #pragma unroll
     for (int i = 0; i < 8; ++i) a[i] = row_f4(rows, (size_t)pa, i * 8 + l8);
     const float inv_na = 1.f / fmaxf(norms[pa], 1e-8f);
     const float scale2 = 1.4426950408889634f / temp;
-    float cur_inv = 1.f / fmaxf(norms[max(cur_row, 0)], 1e-8f);
 
     Online st;
     st.m = FIX ? scale2 : -INFINITY;
@@ -897,7 +913,6 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
     uint32_t parity = 0;
 #pragma unroll 1
     for (int b = 0; b * 8 < T; ++b) {
-        float nxt_nrm = 1.f;
         const bool more = (b + 1) * 8 < T;               // a next batch exists: refills may reach into it
 #pragma unroll 1
         for (int tb0 = 0; tb0 < 8; tb0 += NBUF * PERIOD) {
@@ -905,8 +920,8 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
           for (int ib = 0; ib < NBUF; ++ib) {
             const int t0 = tb0 + ib * PERIOD;
             {   // buffered step
-                const int row = __shfl_sync(0xffffffffu, cur_row, t0 * 4 + grp);
-                const float inv = __shfl_sync(0xffffffffu, cur_inv, t0 * 4 + grp);
+                const int row = __shfl_sync(0xffffffffu, cur.x, t0 * 4 + grp);
+                const float inv = __int_as_float(__shfl_sync(0xffffffffu, cur.y, t0 * 4 + grp));
                 sc_mbar_wait(bar0 + ib * 8, parity);
                 float4 r[8];
 #pragma unroll
@@ -914,15 +929,15 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
                 const float cosv = group_sum8(dot8(a, r)) * (inv_na * inv);
                 __syncwarp();                                   // every lane has read the buffer
                 const int tp = t0 + NBUF * PERIOD;
-                const int prow = __shfl_sync(0xffffffffu, (tp < 8) ? cur_row : nxt_row, (tp & 7) * 4 + grp);
+                const int prow = __shfl_sync(0xffffffffu, (tp < 8) ? cur.x : nxt.x, (tp & 7) * 4 + grp);
                 if (tp < 8 || more) refill(ib, prow);
                 online_update<true, FIX>(st, cosv * scale2, row >= 0, inv, r);
             }
 #pragma unroll
             for (int u = 1; u < PERIOD; ++u) {                  // register steps
                 const int t = t0 + u;
-                const int row = __shfl_sync(0xffffffffu, cur_row, t * 4 + grp);
-                const float inv = __shfl_sync(0xffffffffu, cur_inv, t * 4 + grp);
+                const int row = __shfl_sync(0xffffffffu, cur.x, t * 4 + grp);
+                const float inv = __int_as_float(__shfl_sync(0xffffffffu, cur.y, t * 4 + grp));
                 const float4* p = reinterpret_cast<const float4*>(rows) + (size_t)max(row, 0) * (CSS_D / 4) + l8;
                 float4 r[8];
 #pragma unroll
@@ -930,13 +945,11 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) score_ce_bulk_kernel(
                 const float cosv = group_sum8(dot8(a, r)) * (inv_na * inv);
                 online_update<true, FIX>(st, cosv * scale2, row >= 0, inv, r);
             }
-            if (t0 == 4) nxt_nrm = norms[max(nxt_row, 0)];
           }
           parity ^= 1u;
         }
-        cur_row = nxt_row;
-        cur_inv = 1.f / fmaxf(nxt_nrm, 1e-8f);
-        nxt_row = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, (b + 2) * 32 + lane, cnt);
+        cur = nxt;
+        nxt = ring_candidate_row<FED>(tb, dk, neg_idx, valid_list, k, q, Q, Nn, N, (b + 2) * 32 + lane, cnt);
     }
     finish_query<true, float>(st, z0, cos_pos, sh, rows, proto_hat, inv_na, pa, c, k, q, Q, V, temp, loss_kq, anchor_px, grad_anchor);
 }
@@ -1023,7 +1036,7 @@ extern "C" int css_score_ce(const void* rows, int rows_dtype, const float* norms
     dim3 grid(Q, C);
     // fixed-reference softmax whenever 2^(-2 log2(e)/temp) is far from fp32 underflow (temp > ~0.024); online max otherwise
     const bool fix = (2.f * 1.4426950408889634f / temp) < 120.f;
-#define SC_ARGS(RT_) (const RT_*)rows, norms, (const float4*)proto_hat, class_cdf, valid_list, hard_list, (const int32_t*)meta, anchor_idx, neg_idx, seed, \
+#define SC_ARGS(RT_) (const RT_*)rows, norms, (const float4*)proto_hat, class_cdf, (const int2*)valid_list, hard_list, (const int32_t*)meta, anchor_idx, neg_idx, seed, \
                      N, Q, Nn, temp, loss_kq, anchor_px, (float4*)grad_anchor
 #define SC_RUN(RT_)                                                                                                 \
     do {                                                                                                            \
@@ -1037,7 +1050,7 @@ extern "C" int css_score_ce(const void* rows, int rows_dtype, const float* norms
     } while (0)
     const int path = (grad_anchor && rows_dtype == CSS_DTYPE_F32) ? css_scorer_path() : 0;
     if (path > 0) {
-#define RING_ARGS (const float*)rows, norms, (const float4*)proto_hat, class_cdf, valid_list, hard_list, (const int32_t*)meta, anchor_idx, neg_idx, \
+#define RING_ARGS (const float*)rows, norms, (const float4*)proto_hat, class_cdf, (const int2*)valid_list, hard_list, (const int32_t*)meta, anchor_idx, neg_idx, \
                   seed, N, Q, Nn, temp, loss_kq, anchor_px, (float4*)grad_anchor
 #define RING_RUN(S_, B_) (neg_idx ? (fix ? launch_ring<true, true, S_, B_>(grid, st, RING_ARGS) : launch_ring<false, true, S_, B_>(grid, st, RING_ARGS)) \
                                   : (fix ? launch_ring<true, false, S_, B_>(grid, st, RING_ARGS) : launch_ring<false, false, S_, B_>(grid, st, RING_ARGS)))

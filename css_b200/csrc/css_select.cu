@@ -5,7 +5,8 @@
 //
 // Compaction is a three-kernel stable counting sort (classify+count per 256-pixel tile -> exclusive scan over tiles ->
 // scatter with ballot ranks), because the reference's sampled indices are ranks in row-major order inside each class
-// list (SURVEY.md 7.3-3); an atomic-counter compaction would scramble them.
+// list (SURVEY.md 7.3-3); an atomic-counter compaction would scramble them.  The scatter is a separate entry point
+// (css_select_lists): a valid-list entry carries its pixel's inverse norm, which is final only once the rows are.
 #include "css_common.cuh"
 
 extern "C" int css_select_tiles(int N) { return (N + CSS_SEL_TILE - 1) / CSS_SEL_TILE; }
@@ -149,9 +150,12 @@ __global__ void __launch_bounds__(SCAN_THREADS) select_scan_kernel(int32_t* __re
     }
 }
 
+// valid_list entry = {pixel id, bits of 1 / max(||r||, 1e-8)}: the scorer's one load per candidate, and the same IEEE division
+// it would do (the library builds without fast math), so the bits are those of the division in the scorer
 __global__ void __launch_bounds__(CSS_SEL_TILE) select_scatter_kernel(const uint32_t* __restrict__ valid_bits, const uint32_t* __restrict__ hard_bits,
-                                                                      const int32_t* __restrict__ tile_off, int C, int N, int T,
-                                                                      int32_t* __restrict__ valid_list, int32_t* __restrict__ hard_list) {
+                                                                      const int32_t* __restrict__ tile_off, const float* __restrict__ norms,
+                                                                      int C, int N, int T, int2* __restrict__ valid_list,
+                                                                      int32_t* __restrict__ hard_list) {
     css_pdl_enter();
     __shared__ int wcnt[2][CSS_CMAX][CSS_SEL_TILE / 32];
     __shared__ int toff[2 * CSS_CMAX];             // this tile's offsets of all 2C lists: one round trip, not one per class
@@ -162,6 +166,7 @@ __global__ void __launch_bounds__(CSS_SEL_TILE) select_scatter_kernel(const uint
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t vb = (p < N) ? valid_bits[p] : 0u;
     const uint32_t hb = (p < N) ? hard_bits[p] : 0u;
+    const int inv_bits = vb ? __float_as_int(1.f / fmaxf(norms[p], 1e-8f)) : 0;
     const uint32_t uni = __reduce_or_sync(0xffffffffu, vb);
     for (uint32_t u = uni; u;) {
         const int c = __ffs(u) - 1;
@@ -186,17 +191,15 @@ __global__ void __launch_bounds__(CSS_SEL_TILE) select_scatter_kernel(const uint
             oh += wcnt[1][c][w2];
         }
         if ((vb >> c) & 1u)
-            valid_list[(size_t)c * N + toff[c] + ov + __popc(bv & lt)] = p;
+            valid_list[(size_t)c * N + toff[c] + ov + __popc(bv & lt)] = make_int2(p, inv_bits);
         if ((hb >> c) & 1u)
             hard_list[(size_t)c * N + toff[C + c] + oh + __popc(bh & lt)] = p;
     }
 }
 
 extern "C" int css_select(const float* label, const float* mask, const float* prob, float strong_threshold, int B2, int C,
-                          int h, int w, uint32_t* valid_bits, uint32_t* hard_bits, int32_t* tile_counts, int32_t* valid_list,
-                          int32_t* hard_list, int32_t* meta, void* stream) {
-    CSS_CHECK_ARG(label && mask && prob && valid_bits && hard_bits && tile_counts && valid_list && hard_list && meta, CSS_E_ARG,
-                  "css_select: null pointer");
+                          int h, int w, uint32_t* valid_bits, uint32_t* hard_bits, int32_t* tile_counts, int32_t* meta, void* stream) {
+    CSS_CHECK_ARG(label && mask && prob && valid_bits && hard_bits && tile_counts && meta, CSS_E_ARG, "css_select: null pointer");
     CSS_CHECK_ARG(B2 > 0 && h > 0 && w > 0, CSS_E_ARG, "css_select: non-positive size");
     CSS_CHECK_ARG(C >= 1 && C <= CSS_CMAX, CSS_E_DIM, "css_select: C must be in [1,%d]", CSS_CMAX);
     CSS_CHECK_ARG((long long)B2 * h * w * CSS_CMAX < (1ll << 31), CSS_E_SIZE, "css_select: too many pixels");
@@ -205,8 +208,20 @@ extern "C" int css_select(const float* label, const float* mask, const float* pr
     css_launch(select_classify_kernel, dim3(T), dim3(CSS_SEL_TILE), (size_t)(0), (cudaStream_t)(st), label, mask, prob, strong_threshold, C, hw, N, T, valid_bits, hard_bits,
                                                       tile_counts, meta);
     css_launch(select_scan_kernel, dim3(2 * C), dim3(SCAN_THREADS), (size_t)(0), (cudaStream_t)(st), tile_counts, C, T, meta);
-    css_launch(select_scatter_kernel, dim3(T), dim3(CSS_SEL_TILE), (size_t)(0), (cudaStream_t)(st), valid_bits, hard_bits, tile_counts, C, N, T, valid_list, hard_list);
-    CSS_CHECK_LAUNCH("css_select", 3);
+    CSS_CHECK_LAUNCH("css_select", 2);
+    return 0;
+}
+
+extern "C" int css_select_lists(const uint32_t* valid_bits, const uint32_t* hard_bits, const int32_t* tile_counts, const float* norms,
+                                int C, int N, int32_t* valid_list, int32_t* hard_list, void* stream) {
+    CSS_CHECK_ARG(valid_bits && hard_bits && tile_counts && norms && valid_list && hard_list, CSS_E_ARG, "css_select_lists: null pointer");
+    CSS_CHECK_ARG(N > 0, CSS_E_ARG, "css_select_lists: non-positive size");
+    CSS_CHECK_ARG(C >= 1 && C <= CSS_CMAX, CSS_E_DIM, "css_select_lists: C must be in [1,%d]", CSS_CMAX);
+    CSS_CHECK_ARG((long long)N * CSS_CMAX < (1ll << 31), CSS_E_SIZE, "css_select_lists: too many pixels");
+    const int T = css_select_tiles(N);
+    css_launch(select_scatter_kernel, dim3(T), dim3(CSS_SEL_TILE), (size_t)(0), (cudaStream_t)stream, valid_bits, hard_bits, tile_counts, norms, C, N, T,
+               reinterpret_cast<int2*>(valid_list), hard_list);
+    CSS_CHECK_LAUNCH("css_select_lists", 1);
     return 0;
 }
 

@@ -35,7 +35,7 @@ class _Workspace:
         self.valid_bits = torch.empty(N, **i32)
         self.hard_bits = torch.empty(N, **i32)
         self.tile_counts = torch.empty(2 * C * T, **i32)
-        self.valid_list = torch.empty(C * N, **i32)
+        self.valid_list = torch.empty(C * N * 2, **i32)          # {pixel id, bits of its inverse norm} per entry
         self.hard_list = torch.empty(C * N, **i32)
         self.meta = torch.zeros(_lib.META_WORDS, **i32)
         self.partials = torch.empty(G * C * D, **f32)
@@ -67,8 +67,7 @@ class _ContrastFn(torch.autograd.Function):
         N = ws.N
         st = stream_ptr()
         check(lib.css_select(ptr(label), ptr(mask), ptr(prob), float(mod.strong_threshold), B2, C, h, w, ptr(ws.valid_bits),
-                             ptr(ws.hard_bits), ptr(ws.tile_counts), ptr(ws.valid_list), ptr(ws.hard_list), ptr(ws.meta), st),
-              "css_select")
+                             ptr(ws.hard_bits), ptr(ws.tile_counts), ptr(ws.meta), st), "css_select")
         how = cache.match(rep) if cache is not None else "miss"
         nhwc = is_channels_last(rep)
         if nhwc:                                # channels-last: the map is its own row table; only the norms are carried
@@ -90,6 +89,9 @@ class _ContrastFn(torch.autograd.Function):
         if how == "verify" and not nhwc:        # equal content at another address (DDP's output clone): checked on the device
             check(lib.css_rows_refresh(ptr(rep), rows_dt, ptr(rows), ptr(norms), ptr(ws.meta), B2, D, h, w, st), "css_rows_refresh")
             cache.rebind(rep)
+        # the valid-list entries carry the inverse norms, final only now that the rows are resolved
+        check(lib.css_select_lists(ptr(ws.valid_bits), ptr(ws.hard_bits), ptr(ws.tile_counts), ptr(norms), C, N, ptr(ws.valid_list),
+                                   ptr(ws.hard_list), st), "css_select_lists")
         check(lib.css_class_stats(ptr(rows), rows_dt, ptr(ws.valid_bits), ptr(ws.meta), N, C, D, ptr(ws.partials), ptr(ws.touched),
                                   ptr(ws.class_stats), st), "css_class_stats")
         mod._exchange(ws.class_stats, C, D, dev)
@@ -272,7 +274,7 @@ class Contrast_Loss(nn.Module):
             nv, nh = int(meta[_lib.META_N_VALID + c]), int(meta[_lib.META_N_HARD + c])
             out["num_list"].append(nv)
             out["n_hard"].append(nh)
-            out["valid_ids"].append(ws.valid_list[c * ws.N:c * ws.N + nv].cpu().numpy())
+            out["valid_ids"].append(ws.valid_list[2 * c * ws.N:2 * (c * ws.N + nv):2].cpu().numpy())
             out["hard_ids"].append(ws.hard_list[c * ws.N:c * ws.N + nh].cpu().numpy())
         return out
 

@@ -140,17 +140,23 @@ int css_upsample_label_fuse(const float* sim, const float* logits, float temp, i
 /* ---- stage 3: selection ----------------------------------------------------------------------------------------
  * valid[p,c] = label[p,c]*mask[p] != 0, hard[p,c] = valid && prob[p,c] < strong_threshold, and the ORDER-PRESERVING
  * (row-major) per-class compaction of both.  Replaces loss.py:80,94-99,111-113.
+ * css_select classifies and counts; css_select_lists writes the lists, once the norms of the rows the scorer will read are
+ * final (after css_rep_pass / css_rows_refresh of the same step), because every valid-list entry carries its pixel's inverse norm.
  *   label [B2,C,h,w] f32, mask [B2,1,h,w] f32, prob [B2,C,h,w] f32          N = B2*h*w
  *   valid_bits, hard_bits   u32[N]      per-pixel class sets
- *   tile_counts             i32[2*C*T]  scratch, T = css_select_tiles(N)
- *   valid_list, hard_list   i32[C*N]    class c's pixel ids start at c*N (fixed stride, no cross-class scan)
+ *   tile_counts             i32[2*C*T]  scratch, T = css_select_tiles(N); css_select leaves the lists' tile offsets in it
  *   meta                    i32[CSS_META_WORDS]   counts / present classes, layout CSS_META_*
+ *   norms                   f32[N]      ||r_p|| (from css_rep_pass / css_rep_pass_nhwc / css_rows_refresh)
+ *   valid_list              i32[C*N*2]  entry (c*N + i) = {pixel id, bits of the f32 1 / max(norms[id], 1e-8)}: class c's
+ *                                       entries start at c*N (fixed stride, no cross-class scan)
+ *   hard_list               i32[C*N]    class c's pixel ids start at c*N
  */
 int css_select_tiles(int N);
 int css_select(const float* label, const float* mask, const float* prob, float strong_threshold,
                int B2, int C, int h, int w,
-               uint32_t* valid_bits, uint32_t* hard_bits, int32_t* tile_counts,
-               int32_t* valid_list, int32_t* hard_list, int32_t* meta, void* stream);
+               uint32_t* valid_bits, uint32_t* hard_bits, int32_t* tile_counts, int32_t* meta, void* stream);
+int css_select_lists(const uint32_t* valid_bits, const uint32_t* hard_bits, const int32_t* tile_counts, const float* norms,
+                     int C, int N, int32_t* valid_list, int32_t* hard_list, void* stream);
 
 /* ---- stage 4a: per-class statistics ----------------------------------------------------------------------------------
  * Per-class feature sums and counts of this rank from the pixel-major rows: the all-reduce payload that replaces the
@@ -192,7 +198,8 @@ int css_sample(const int32_t* meta, const float* class_cdf, uint64_t seed, uint6
                int32_t* anchor_idx, int32_t* neg_idx, void* stream);
 
 /* ---- stage 3: scoring + cross-entropy + d loss / d anchor ------------------------------------------------------------
- * Replaces loss.py:124-149 and its autograd backward up to the anchor rows.  rows / norms come from css_rep_pass.
+ * Replaces loss.py:124-149 and its autograd backward up to the anchor rows.  rows / norms come from css_rep_pass, valid_list /
+ * hard_list from css_select_lists with the same norms (norms itself is read for the anchors only).
  *   anchor_idx / neg_idx: as produced by css_sample or recorded from the reference; NULL = draw on the fly with
  *   (seed, offset + *step_counter), bit-identical to css_sample with the same (seed, offset).
  *   step_counter: optional DEVICE u64, read as an offset increment and incremented by one by the call, so that replays of a

@@ -6,11 +6,20 @@
 // Each runs at 16, 20 and 24 warps/SM (launch bound + padding shared memory), with no math ("load": the rows are only summed)
 // or with a stub of the scorer's per-row work ("stub"): the dot with a register anchor, its reduction (group: 3 shuffles; wide:
 // the batched transpose-reduce), one exp2, the weight broadcast and the accumulation into a register gradient slice.
+// `dev_gather_wide ids` runs only the candidate-id comparison (wide R = 8, one batch, 16 warps/SM, with the stub), in three
+// ways of getting a batch's row ids and inverse norms:
+//   (a) ids read contiguously, as above, inverse norm 1;
+//   (b) per candidate a random 4-byte id from a class list, then a dependent 4-byte norm load and 1 / max(norm, 1e-8)
+//       (IEEE division), the norm of the next 32 ids loaded after the batch's first rows, as score_rows_wide did;
+//   (c) per candidate one random 8-byte {id, bits of the inverse norm} list entry.
+// The list positions are random (they stand in for the scorer's Philox draws); the stub scales each dot and weight by the
+// inverse norm, so no load is dead.  Five alternating rounds of the three.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -Xptxas -v -o dev_gather_wide dev_gather_wide.cu
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <string.h>
 
 #define N_WARPS 5376
 #define PER_WARP 512
@@ -167,16 +176,79 @@ __global__ void __launch_bounds__(128, MINB) wide_kernel(const float4* __restric
     if (s == 123.456f) out[0] = s + pad[0];
 }
 
+// ---- candidate ids (whole-warp rows, R = 8, one batch, stub) -------------------------------------------------------------
+template <int MODE>
+__device__ __forceinline__ int batch_ids(const int* __restrict__ list, const float* __restrict__ norms, const int2* __restrict__ entries,
+                                         int pos, float& inv) {
+    if (MODE == 0) { inv = 1.f; return pos; }
+    if (MODE == 1) { const int id = list[pos]; inv = 1.f / fmaxf(norms[id], 1e-8f); return id; }
+    const int2 e = entries[pos];
+    inv = __int_as_float(e.y);
+    return e.x;
+}
+
+template <int MODE, int MINB>
+__global__ void __launch_bounds__(128, MINB) ids_kernel(const float4* __restrict__ rows, const int* __restrict__ idx, const int* __restrict__ list,
+                                                        const float* __restrict__ norms, const int2* __restrict__ entries, float* __restrict__ out) {
+    extern __shared__ float pad[];
+    constexpr int R = 8, LPR = 32 / R;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    const int* my = idx + (size_t)warp * PER_WARP;
+    const float4 a0 = rows[(size_t)warp * 64 + lane], a1 = rows[(size_t)warp * 64 + 32 + lane];
+    float4 acc0 = make_float4(0.f, 0.f, 0.f, 0.f), acc1 = acc0;
+    float l = 0.f, cur_inv;
+    int cur = batch_ids<MODE>(list, norms, entries, my[lane], cur_inv);
+#pragma unroll 1
+    for (int b = 0; b < PER_WARP; b += 32) {
+        const int pos = (b + 32 < PER_WARP) ? my[b + 32 + lane] : 0;
+        int nxt;
+        float nxt_inv = 1.f, nxt_nrm = 1.f;
+        if (MODE == 1) nxt = list[pos];                           // its norm is loaded after the batch's first rows
+        else nxt = batch_ids<MODE>(list, norms, entries, pos, nxt_inv);
+#pragma unroll 1
+        for (int t = 0; t < 32; t += R) {
+            float4 r[R][2];
+            load_rows<R>(rows, cur, t, lane, r);
+            float d[R];
+#pragma unroll
+            for (int i = 0; i < R; ++i) {
+                float2 s = __fmul2_rn(lo2(a0), lo2(r[i][0]));
+                s = __ffma2_rn(hi2(a0), hi2(r[i][0]), s);
+                s = __ffma2_rn(lo2(a1), lo2(r[i][1]), s);
+                s = __ffma2_rn(hi2(a1), hi2(r[i][1]), s);
+                d[i] = s.x + s.y;
+            }
+            const float inv = __shfl_sync(0xffffffffu, cur_inv, t + lane / LPR);
+            const float w = exp2f(transpose_sum<R>(d, lane) * inv * 1e-3f - 2.f);
+            if (lane % LPR == 0) l += w;
+            const float wr = w * inv;
+#pragma unroll
+            for (int i = 0; i < R; ++i) {
+                const float wi = __shfl_sync(0xffffffffu, wr, i * LPR);
+                axpy4(wi, r[i][0], acc0);
+                axpy4(wi, r[i][1], acc1);
+            }
+            if (MODE == 1 && t == 0) nxt_nrm = norms[nxt];
+        }
+        cur = nxt;
+        cur_inv = (MODE == 1) ? 1.f / fmaxf(nxt_nrm, 1e-8f) : nxt_inv;
+    }
+    const float s = l + sum4(acc0) + sum4(acc1);
+    if (s == 123.456f) out[0] = s + pad[0];
+}
+
 // ---- driver --------------------------------------------------------------------------------------------------------------
 typedef void (*Kern)(const float4*, const int*, float*);
 
-static double run(Kern k, int target_ctas, const char* name, const float4* rows, const int* idx, float* out, double clk_ghz, int n_sm) {
+// `launch(smem)` launches kernel `kf` once with that much padding shared memory
+template <typename Launch>
+static double run_kernel(const void* kf, Launch launch, int target_ctas, const char* name, double clk_ghz, int n_sm) {
     cudaFuncAttributes fa;
-    cudaFuncGetAttributes(&fa, k);
+    cudaFuncGetAttributes(&fa, kf);
     int smem = 0, occ = 0;
     for (smem = 0; smem <= 200 * 1024; smem += 512) {         // the least padding that leaves target_ctas CTAs per SM
-        cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, 128, smem);
+        cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kf, 128, smem);
         if (occ <= target_ctas) break;
     }
     cudaEvent_t e0, e1;
@@ -185,7 +257,7 @@ static double run(Kern k, int target_ctas, const char* name, const float4* rows,
     float best = 1e30f;
     for (int rep = 0; rep < 5; ++rep) {
         cudaEventRecord(e0);
-        k<<<N_WARPS / 4, 128, smem>>>(rows, idx, out);
+        launch(smem);
         cudaEventRecord(e1);
         cudaEventSynchronize(e1);
         float ms;
@@ -201,7 +273,19 @@ static double run(Kern k, int target_ctas, const char* name, const float4* rows,
     return tbs;
 }
 
-int main() {
+static double run(Kern k, int target_ctas, const char* name, const float4* rows, const int* idx, float* out, double clk_ghz, int n_sm) {
+    return run_kernel((const void*)k, [&](int smem) { k<<<N_WARPS / 4, 128, smem>>>(rows, idx, out); }, target_ctas, name, clk_ghz, n_sm);
+}
+
+typedef void (*IdsKern)(const float4*, const int*, const int*, const float*, const int2*, float*);
+static double run_ids(IdsKern k, const char* name, const float4* rows, const int* idx, const int* list, const float* norms,
+                      const int2* entries, float* out, double clk_ghz, int n_sm) {
+    return run_kernel((const void*)k, [&](int smem) { k<<<N_WARPS / 4, 128, smem>>>(rows, idx, list, norms, entries, out); }, 4, name,
+                      clk_ghz, n_sm);
+}
+
+int main(int argc, char** argv) {
+    const bool ids_only = argc > 1 && !strcmp(argv[1], "ids");
     const int n_rows = 104976;
     float4* rows;
     int* idx;
@@ -238,6 +322,37 @@ int main() {
     run(wide_kernel<STUB, 8, true, 4>, 4, "wide R8 halves " TAG, rows, idx, out, ghz, n_sm);                                   \
     run(wide_kernel<STUB, 8, true, 5>, 5, "wide R8 halves " TAG, rows, idx, out, ghz, n_sm);                                   \
     run(wide_kernel<STUB, 8, true, 6>, 6, "wide R8 halves " TAG, rows, idx, out, ghz, n_sm)
+    if (ids_only) {
+        // list[p]: a row id; norms in [0.5, 2); entries[p] = {list[p], bits of 1 / max(norms[list[p]], 1e-8)}
+        int* hl = (int*)malloc((size_t)n_rows * 4);
+        float* hn = (float*)malloc((size_t)n_rows * 4);
+        int2* he = (int2*)malloc((size_t)n_rows * 8);
+        for (int i = 0; i < n_rows; ++i) hn[i] = 0.5f + 1.5f * (float)rand() / (float)RAND_MAX;
+        for (int i = 0; i < n_rows; ++i) {
+            hl[i] = (int)(((uint64_t)rand() * 2654435761u) % n_rows);
+            const float inv = 1.f / fmaxf(hn[hl[i]], 1e-8f);
+            int bits;
+            memcpy(&bits, &inv, 4);
+            he[i] = make_int2(hl[i], bits);
+        }
+        int* dl;
+        float* dn;
+        int2* de;
+        cudaMalloc(&dl, (size_t)n_rows * 4);
+        cudaMalloc(&dn, (size_t)n_rows * 4);
+        cudaMalloc(&de, (size_t)n_rows * 8);
+        cudaMemcpy(dl, hl, (size_t)n_rows * 4, cudaMemcpyHostToDevice);
+        cudaMemcpy(dn, hn, (size_t)n_rows * 4, cudaMemcpyHostToDevice);
+        cudaMemcpy(de, he, (size_t)n_rows * 8, cudaMemcpyHostToDevice);
+        for (int round = 0; round < 5; ++round) {
+            printf("round %d\n", round);
+            run_ids(ids_kernel<0, 4>, "ids (a) contiguous", rows, idx, dl, dn, de, out, ghz, n_sm);
+            run_ids(ids_kernel<1, 4>, "ids (b) list + norm + div", rows, idx, dl, dn, de, out, ghz, n_sm);
+            run_ids(ids_kernel<2, 4>, "ids (c) 8-byte entry", rows, idx, dl, dn, de, out, ghz, n_sm);
+        }
+        printf("last error: %s\n", cudaGetErrorString(cudaDeviceSynchronize()));
+        return 0;
+    }
     ALL(false, "load");
     ALL(true, "stub");
     printf("last error: %s\n", cudaGetErrorString(cudaDeviceSynchronize()));

@@ -72,11 +72,14 @@ def main():
     D = 256
     B2 = 2 * B
 
+    rows, norms = crit.last["rows"], crit.last["norms"]
+
     def select(i):
         check(lib.css_select(ptr(label), ptr(mask), ptr(prob), float(cfg["strong"]), B2, C, h, w, ptr(ws.valid_bits), ptr(ws.hard_bits),
-                             ptr(ws.tile_counts), ptr(ws.valid_list), ptr(ws.hard_list), ptr(ws.meta), stream_ptr()), "select")
+                             ptr(ws.tile_counts), ptr(ws.meta), stream_ptr()), "select")
+        check(lib.css_select_lists(ptr(ws.valid_bits), ptr(ws.hard_bits), ptr(ws.tile_counts), ptr(norms), C, N, ptr(ws.valid_list),
+                                   ptr(ws.hard_list), stream_ptr()), "select_lists")
 
-    rows, norms = crit.last["rows"], crit.last["norms"]
     rows_dt = 1 if rows.dtype == torch.bfloat16 else 0
 
     def stream(i):
